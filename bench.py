@@ -8,7 +8,7 @@ A *step* is one pass of the hot path (PhysicsEnv.step: act -> physics -> reward 
 done / auto-reset -> observation) over every env of the batch: ONE kernel launch.
 Workload (BASELINE.json config 3, the throughput config; weak scaling): Balance-v0
 (gym/optimized_walker.py:176-199), in3d, 2^20 envs per GPU, U(-1,1) float32
-actions resident on the device, template auto-reset, reference semantics as written.
+actions resident on the device, template auto-reset after EPISODE_STEPS env-steps, reference semantics as written.
 Rank 0 prints ONE JSON line.  Besides the headline it carries short sub-measurements of
 the other BASELINE configs (`sub_configs`), the end-to-end number on host buffers (`e2e`)
 next to the box's own device-to-host ceiling measured in the same run, the roofline of
@@ -34,8 +34,12 @@ UNIT = "env-steps/s"
 ENV_ID = "Balance-v0"
 N_MASS, N_MUSCLE = 4, 2
 OBS_DIM = 3 * 3 * N_MASS + N_MUSCLE
-PREROLL = 256          # untimed env-steps before any timed window: the timed region is the steady state, not the
-#                        first steps after a template reset (every env finite, no divergent non-finite lanes)
+ROLLOUT_T = 32         # config 5: env-steps per RolloutCollector.collect (one CUDA-graph replay)
+PREROLL = 256          # untimed env-steps before any timed window: the timed region is the steady state of the reset
+#                        cycle, not the first steps after the initial template reset
+EPISODE_STEPS = 30     # max_steps of every config 3 measurement and of its CPU arms: Balance-v0's as-written dynamics
+#                        overflow float32 no sooner than ~34 env-steps after a reset, so every env stepped stays finite
+#                        (with the reference's default of 1000, ~70 % of the envs hold inf / NaN in steady state)
 
 
 def algorithmic_bytes(n_mass: int, n_muscle: int) -> int:
@@ -80,7 +84,18 @@ def parse():
     ap.add_argument("--no-affinity", action="store_true", help="do not bind the rank to CPUs next to its GPU")
     ap.add_argument("--strong-envs-per-gpu", type=int, default=0,
                     help="sub-config 3_strong: envs per GPU (default 2^20 / n_gpus, BASELINE config 3 as written)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed window, write rank 0's results of the last timed step (obs, reward, done) "
+                         "as DIR/<name>.npy in float32; above 63 MB in all, every array keeps the same seeded sample of envs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.config == 5 and args.steps % ROLLOUT_T:
+        ap.error(f"--config 5 times whole {ROLLOUT_T}-step rollouts: --steps must be a multiple of {ROLLOUT_T}")
+    if args.dump_outputs and (args.impl != "ours" or args.probe_stream or args.config != 3 or args.body != "balance"
+                              or args.steps_per_launch > 1 or args.k_sub > 1):
+        ap.error("--dump-outputs applies to the headline path (--config 3, --body balance, one env-step per launch)")
+    return args
 
 
 def hbm_peak():
@@ -167,7 +182,7 @@ def cpu_run(n_env: int, steps: int, warmup: int, seed: int = 0):
     import walker_oracle as wo
     threads = wo.set_threads(len(host_cpus()))      # all host threads (torchrun would pin OMP_NUM_THREADS=1)
     body = wo.make_body(wo.BALANCE)
-    prm = wo.make_params(in3d=True, auto_reset=2, seed=seed)
+    prm = wo.make_params(in3d=True, auto_reset=2, seed=seed, max_steps=EPISODE_STEPS)
     st = wo.init_state(body, n_env)
     st.pop("old_a")
     wo.reset(body, prm, st, mode=2)
@@ -226,7 +241,9 @@ def _ref_worker(idx, cpu, ref_root, n_warm, n_timed, barrier, out_q):
     def make():
         engine.Point.clear()
         np.random.seed(idx)
-        return envmod.make_env(ENV_ID, in3d=True)
+        env = envmod.make_env(ENV_ID, in3d=True)
+        env.max_steps = EPISODE_STEPS
+        return env
 
     env = make()
     done_steps = 0
@@ -297,7 +314,8 @@ def run_reference(args):
         sample = (f"the unmodified reference modules (bytecode in {ref['ref_root']}, oracle/make_ref.py) through their own "
                   f"make_env / PhysicsEnv.step, {ENV_ID} in3d: {cores} processes (one env each: the reference's Point "
                   f"registry is process-global), {ref['per_step']} env.step calls per bench step and process, "
-                  f"{ref['total_env_steps']} env-steps in {dt:.1f} s; float32 U(-1,1) actions, make_env again on done")
+                  f"{ref['total_env_steps']} env-steps in {dt:.1f} s; float32 U(-1,1) actions, make_env again on done "
+                  f"(max_steps = {EPISODE_STEPS})")
         workload = (f"{ENV_ID} in3d=True, template auto-reset, U(-1,1) f32 actions; reference arm: one env per process on "
                     f"{cores} host cores, a bench step = {ref['per_step']} env.step calls per process (the GPU arm steps "
                     "2^20 envs per GPU per step)")
@@ -389,6 +407,27 @@ def action_ring(ctx, E, M, n=16, seed=100):
     return [(torch.rand(E, M, device=ctx.dev, generator=g) * 2 - 1) for _ in range(n)]
 
 
+DUMP_BYTES = 63 * 10 ** 6      # a dump stays under 64 MB with its .npy headers
+
+
+def dump_outputs(directory: str, outputs: dict, n_envs: int):
+    """Write ``outputs`` ({name: (tensor, env axis)}) as ``directory/<name>.npy`` in float32.  If they do not fit in
+    DUMP_BYTES, each keeps the envs of one fixed sample (seed 0, env order), so that two builds compare output for output."""
+    import numpy as np
+    import torch
+    per_env = 4 * sum(t.numel() // n_envs for t, _ in outputs.values())
+    keep = min(n_envs, DUMP_BYTES // per_env)
+    idx = None
+    if keep < n_envs:
+        idx = torch.from_numpy(np.sort(np.random.default_rng(0).choice(n_envs, keep, replace=False)))
+    os.makedirs(directory, exist_ok=True)
+    for name, (t, axis) in outputs.items():
+        t = t.float()
+        if idx is not None:
+            t = t.index_select(axis, idx.to(t.device))
+        np.save(os.path.join(directory, name + ".npy"), t.cpu().numpy())
+
+
 def run_ours(args):
     ctx = Ctx(args)
     torch = ctx.torch
@@ -413,8 +452,9 @@ def run_ours(args):
     if args.k_sub > 0:
         k_sub = args.k_sub
 
+    max_steps = EPISODE_STEPS if args.config == 3 else 1000     # config 4: the reference's default
     env = BatchedPhysicsEnv(body, E, dev, in3d=True, auto_reset="template", seed=1234, env_offset=rank * E,
-                            track_stats=True, k_sub=k_sub, obs_layout=args.obs_layout)
+                            track_stats=True, k_sub=k_sub, obs_layout=args.obs_layout, max_steps=max_steps)
     bytes_per_env_step = algorithmic_bytes(env.N, env.M)
     ring = action_ring(ctx, E, env.M)
 
@@ -428,8 +468,12 @@ def run_ours(args):
     for t in range(W):
         env.step(ring[t % 16])
     ms, clocks = ctx.timed(lambda t: env.step(ring[t % 16]), K, clocks=True)
+    if args.dump_outputs and rank == 0:
+        # env.step returns views of these buffers: they hold the last timed step's results until the next step
+        dump_outputs(args.dump_outputs, {"obs": (env.obs, 0 if args.obs_layout == "row" else 1),
+                                         "reward": (env.reward, 0), "done": (env.done, 0)}, E)
     value = world * E * K / (ms * 1e-3)
-    # one whole episode period (max_steps = 1000 env-steps: ~50 finite steps, then non-finite lanes until the reset)
+    # a longer window right after the timed one
     long_n = 1000 if env.N <= 8 and k_sub == 1 else 100
     ms_long = ctx.timed(lambda t: env.step(ring[t % 16]), long_n)
     stats = env.episode_stats(all_reduce=True)       # the only collective: 8 doubles, off the timed path
@@ -460,7 +504,7 @@ def run_ours(args):
             "dtype": "f32", "data": "synthetic",
             "config": {"workload": f"{body}" + (" (gym/optimized_walker.py create_balance_creature)" if args.body == "balance" else "") +
                                    f", in3d=True, {E} envs per GPU, 1 kernel launch per env-step, K_sub={k_sub}, template "
-                                   "auto-reset, reference semantics as written, U(-1,1) f32 actions from a 16-deep device ring; "
+                                   f"auto-reset at max_steps = {max_steps}, reference semantics as written otherwise, U(-1,1) f32 actions from a 16-deep device ring; "
                                    f"{PREROLL} untimed pre-roll env-steps + {W} warm-up steps before the timed window (steady state)",
                        "baseline_config": args.config,
                        "envs_per_gpu": E, "global_envs": world * E, "state_layout": env.state_layout, "obs": (f"row-major [E,{env.obs_dim}] materialised" if args.obs_layout == "row"
@@ -476,7 +520,7 @@ def run_ours(args):
                          "window": f"{K} steps after {PREROLL} pre-roll + {W} warm-up steps",
                          "episode_period": {"steps": long_n, "kernel_us": ms_long * 1e3 / long_n,
                                             "frac": E * bytes_per_env_step / (ms_long * 1e-3 / long_n) / 1e9 / peak,
-                                            "what": "average over one whole episode period (max_steps = 1000) right after the timed window"},
+                                            "what": f"average over {long_n} env-steps right after the timed window (max_steps = {max_steps})"},
                          "early_episode": {"steps": 20, "kernel_us": ms_early * 1e3 / 20,
                                            "frac": E * bytes_per_env_step / (ms_early * 1e-3 / 20) / 1e9 / peak,
                                            "what": "the first steps after a template reset (every lane finite): NOT the headline"}},
@@ -653,7 +697,7 @@ def measure_sub_configs(ctx, args):
     def strong():
         Es = args.strong_envs_per_gpu or (1 << 20) // world
         env = BatchedPhysicsEnv(ENV_ID, Es, dev, in3d=True, auto_reset="template", seed=1234, env_offset=rank * Es,
-                                track_stats=True, graph_safe=True)
+                                track_stats=True, graph_safe=True, max_steps=EPISODE_STEPS)
         T = 50
         g = torch.Generator(device=dev).manual_seed(300 + rank)
         acts = torch.rand(T, Es, env.M, device=dev, generator=g) * 2 - 1
@@ -683,7 +727,8 @@ def measure_sub_configs(ctx, args):
         ms_p = ctx.timed(lambda i: pg.replay(), n_rep)
         us_p = ms_p * 1e3 / (n_rep * T)
         return {"what": f"BASELINE config 3 as written: 2^20 envs in total = {Es} per GPU x {world} GPU(s), {n_rep * T}-step "
-                        f"closed-loop rollout, {T} wg_step launches per CUDA-graph replay (StepGraph), template auto-reset",
+                        f"closed-loop rollout, {T} wg_step launches per CUDA-graph replay (StepGraph), template auto-reset "
+                        f"at max_steps = {EPISODE_STEPS}",
                 "scaling": "strong", "envs_per_gpu": Es, "steps": n_rep * T, "kernel_us": us,
                 "value": world * Es / (us * 1e-6), "unit": UNIT,
                 "frac_hbm": Es * b / (us * 1e-6) / 1e9 / peak,
@@ -719,7 +764,7 @@ def measure_sub_configs(ctx, args):
     def multi():
         E, T = args.envs_per_gpu, 16
         env = BatchedPhysicsEnv(ENV_ID, E, dev, in3d=True, auto_reset="template", seed=1234, env_offset=rank * E,
-                                track_stats=True, state_layout="packed")
+                                track_stats=True, state_layout="packed", max_steps=EPISODE_STEPS)
         g = torch.Generator(device=dev).manual_seed(500 + rank)
         ring = [(torch.rand(T, E, env.M, device=dev, generator=g) * 2 - 1) for _ in range(2)]
         res = (torch.empty(T, E, device=dev), torch.empty(T, E, dtype=torch.uint8, device=dev))
@@ -776,7 +821,7 @@ def run_multi(args, ctx):
     W, K, E, T = max(args.warmup, 3), args.steps, args.envs_per_gpu, args.steps_per_launch
     env_id = {"balance": ENV_ID, "box": "Box-v0", "legacy_box": "box"}.get(args.body, args.body)
     env = BatchedPhysicsEnv(env_id, E, dev, in3d=True, auto_reset="template", seed=1234, env_offset=rank * E,
-                            track_stats=True, k_sub=args.k_sub or 1, state_layout="packed")
+                            track_stats=True, k_sub=args.k_sub or 1, state_layout="packed", max_steps=EPISODE_STEPS)
     g = torch.Generator(device=dev).manual_seed(100 + rank)
     ring = [(torch.rand(T, E, env.M, device=dev, generator=g) * 2 - 1) for _ in range(4)]
     out = (torch.empty(T, E, device=dev), torch.empty(T, E, dtype=torch.uint8, device=dev))
@@ -836,7 +881,7 @@ def run_multi(args, ctx):
                 "dtype": "f32", "data": "synthetic",
                 "config": {"workload": f"{env_id}, in3d=True, {E} envs per GPU, {T} env-steps per launch (wg_step_multi: actions "
                                        f"[T,E,M] known up front, per-step reward / done, observation after the last step), "
-                                       "template auto-reset, U(-1,1) f32 actions from a 4-deep device ring of blocks",
+                                       f"template auto-reset at max_steps = {EPISODE_STEPS}, U(-1,1) f32 actions from a 4-deep device ring of blocks",
                            "baseline_config": "next row f2", "envs_per_gpu": E, "global_envs": world * E,
                            "steps_per_launch": T, "us_per_env_step": per_launch_s * 1e6 / T,
                            "l2": f"state+obs+actions per launch = {E * bytes_per_launch_env / 1e6:.0f} MB > 126 MB L2"},
@@ -911,7 +956,7 @@ def run_rollout(args, ctx):
     from walker_gym_b200.rollout import FeatureMajorMLP, RolloutCollector
     rank, world, dev = ctx.rank, ctx.world, ctx.dev
     E = args.envs_per_gpu if args.envs_per_gpu != (1 << 20) else (1 << 18)
-    T = 32
+    T = ROLLOUT_T
     torch.manual_seed(7 + rank)
     fused = args.policy != "torch"
     lay = "row" if (fused and args.obs_layout == "row") else "feature"
@@ -919,7 +964,7 @@ def run_rollout(args, ctx):
                             obs_layout=lay, act_layout=lay, graph_safe=True)
     pol = FeatureMajorMLP(env.obs_dim, env.M).to(dev)
     col = RolloutCollector(env, pol, T, fused=fused, precision="tf32" if args.policy == "fused-tf32" else "fp32")
-    n_roll = max(1, args.steps // T)
+    n_roll = args.steps // T
     n_warm = max(3, args.warmup // T, PREROLL // T)
     for _ in range(n_warm):
         col.collect()

@@ -11,7 +11,8 @@ for p in (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")):
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs the read-only reference checkout at /root/reference")
+    config.addinivalue_line("markers", "reference: compares with a checkout of the original walker-gym project, found "
+                                       "through WALKER_GYM_REFERENCE; skips without one")
 
 
 def _has_gpu():

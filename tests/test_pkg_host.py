@@ -133,13 +133,14 @@ def test_env_state_rejects_foreign_classes(tmp_path):
 @pytest.mark.reference
 def test_reference_reads_env_state_we_write(tmp_path):
     """The reference's own Environment.load_state accepts a file written by save_state."""
-    if not os.path.isdir("/root/reference/gym/optimized_walker"):
+    import ref_harness_l2 as r2
+    if not r2.available():
         pytest.skip("reference checkout not present")
     env, _ = build("leg2", ground_level=-30)
     out = tmp_path / "env_state.pkl"
     env.save_state(str(out))
     code = ("import sys\nfrom unittest import mock\nsys.modules['pygame'] = mock.MagicMock()\n"
-            "sys.path.insert(0, '/root/reference/gym')\nfrom optimized_walker.env import Environment\n"
+            f"sys.path.insert(0, {os.path.join(r2.DEFAULT_REF, 'gym')!r})\nfrom optimized_walker.env import Environment\n"
             f"e = Environment(); e.load_state({str(out)!r})\n"
             "e.update_physics()\n"
             "print(len(e.points), len(e.springs), e.ground_level, type(e.points[0]).__module__)\n")
