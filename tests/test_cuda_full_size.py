@@ -29,9 +29,10 @@ def n_sms():
     return torch.cuda.get_device_properties(0).multi_processor_count
 
 
-def default_slices(E, n=SLICE):
-    """Head, tail, and a slice across the end of the first wave of CTAs (MIN_BLOCKS per SM) when it is clear of both."""
-    wave = MIN_BLOCKS * n_sms() * PACKED_BLOCK
+def default_slices(E, n=SLICE, block=PACKED_BLOCK, per_sm=MIN_BLOCKS):
+    """Head, tail, and a slice across the end of the first wave of CTAs (`per_sm` CTAs of `block` envs per SM) when it
+    is clear of both."""
+    wave = per_sm * n_sms() * block
     out = [(0, min(n, E))]
     if E > n:
         out.append((E - n, E))
@@ -51,30 +52,40 @@ def _where(a, b):
 
 
 class SliceLockstep:
-    """One oracle state per env slice [a, a + n) of a Balance-v0 env, built with env_offset = a; the env and the oracle
-    start from the same template reset (Philox step index 0), so step k of the run has step index k + 1."""
+    """One oracle state per env slice [a, a + n) of an env, built with env_offset = a; the env and the oracle start
+    from the same initial reset (Philox step index 0), so step k of the run has step index k + 1.  The defaults are
+    bench.py's config 3 (Balance-v0, one substep, template auto-reset, the packed kernel's 128-env CTAs); `block` is
+    the step kernel's envs per CTA (failure messages name CTAs with it).  With `gen` (a wo.gen_actions description)
+    the oracle takes each step's actions from the in-kernel action source instead of from the recorded device
+    actions."""
 
-    def __init__(self, env, slices, *, max_steps, seed):
+    def __init__(self, env, slices, *, max_steps, seed, spec=wo.BALANCE, k_sub=1, auto_reset="template",
+                 rand_sigma=0.1, in3d=True, block=PACKED_BLOCK, gen=None):
         import torch
-        assert env.obs_layout == "row" and env.in3d and env.num_envs >= max(b for _, b in slices)
+        assert env.obs_layout == "row" and env.in3d == in3d and env.num_envs >= max(b for _, b in slices)
         self.env, self.slices, self.step_index = env, list(slices), 1
-        self._max_steps, self._seed = max_steps, seed
-        self.body = wo.make_body(wo.BALANCE)
+        self.block, self.gen = block, gen
+        mode = {"jitter": 1, "template": 2}[auto_reset]
+        self._prm_kw = dict(in3d=in3d, auto_reset=mode, max_steps=int(max_steps), k_sub=k_sub, rand_sigma=rand_sigma,
+                            seed=seed)
+        self.body = wo.make_body(spec)
         self.track = env.fin_stats is not None
         self.parts = []
         for a, b in self.slices:
-            prm = wo.make_params(in3d=True, auto_reset=2, max_steps=max_steps, seed=seed, env_offset=a)
+            prm = wo.make_params(env_offset=a, **self._prm_kw)
             st = wo.init_state(self.body, b - a)
             if env.old_a is None:
                 st.pop("old_a")
             prm.step_index = 0
-            o = wo.reset(self.body, prm, st, mode=2)
+            o = wo.reset(self.body, prm, st, mode=mode)
             ep = (np.zeros(b - a, np.float32), np.zeros((4, b - a), np.float32)) if self.track else (None, None)
             self.parts.append((a, b, prm, st, ep, o))
         self.idx = torch.cat([torch.arange(a, b, device=env.obs.device) for a, b in self.slices])
         self._pending = []
         self.nonfinite = 0               # obs rows of the slices seen non-finite so far
         self.done_count = 0
+        self.obs_rows = 0                # obs rows compared so far, and how many of them were entirely finite
+        self.finite_rows = 0
         self.check_obs(env.obs, "reset")
 
     def _split(self, t):
@@ -85,10 +96,9 @@ class SliceLockstep:
         return out
 
     def _msg(self, a, what, where):
-        E, b = self.env.num_envs, dict(self.slices)[a]
-        n_blocks = (E + PACKED_BLOCK - 1) // PACKED_BLOCK
-        return (f"{what}: slice [{a}, {b}) of {E} envs = CTAs [{a // PACKED_BLOCK}, {(b - 1) // PACKED_BLOCK}] of "
-                f"{n_blocks}: {where}")
+        E, b, B = self.env.num_envs, dict(self.slices)[a], self.block
+        n_blocks = (E + B - 1) // B
+        return f"{what}: slice [{a}, {b}) of {E} envs = CTAs [{a // B}, {(b - 1) // B}] of {n_blocks}: {where}"
 
     def restrict(self, slices):
         """Continue with sub-slices of a lockstep that follows the whole batch [0, E) (cheaper from here on)."""
@@ -97,16 +107,21 @@ class SliceLockstep:
         assert (a0, b0) == (0, self.env.num_envs)
         self.slices, self.parts = list(slices), []
         for a, b in self.slices:
-            prm = wo.make_params(in3d=True, auto_reset=2, max_steps=int(self._max_steps), seed=self._seed, env_offset=a)
+            prm = wo.make_params(env_offset=a, **self._prm_kw)
             sub = {k: np.ascontiguousarray(v[..., a:b]) for k, v in st.items()}
             sep = (ep[0][a:b].copy(), np.ascontiguousarray(ep[1][:, a:b])) if self.track else (None, None)
             self.parts.append((a, b, prm, sub, sep, o[a:b]))
         self.idx = torch.cat([torch.arange(a, b, device=self.env.obs.device) for a, b in self.slices])
 
+    def _count_obs(self, want):
+        self.obs_rows += want.shape[0]
+        self.finite_rows += int(np.isfinite(want).all(1).sum())
+
     def check_obs(self, obs, what):
         got = self._split(obs[self.idx].cpu().numpy())
         for (a, b, prm, st, ep, o), g in zip(self.parts, got):
             assert gu.same(g, o), self._msg(a, f"obs {what}", _where(g, o))
+            self._count_obs(o)
 
     def record(self, action, obs=None, reward=None, done=None):
         """Gather the slice rows of the step the env has just been given -- its device actions [E, M] and results obs
@@ -123,14 +138,17 @@ class SliceLockstep:
         host = [{k: None if v is None else v.cpu().numpy() for k, v in r.items()} for r in pending]
         out_steps = []
         for got in host:
-            acts = self._split(got["action"])
+            acts = None if self.gen is not None else self._split(got["action"])
             split = {k: None if got[k] is None else self._split(got[k]) for k in ("obs", "reward", "done")}
             for p, (a, b, prm, st, ep, _) in enumerate(self.parts):
                 prm.step_index = self.step_index
-                out = wo.step(self.body, prm, st, acts[p], want_info=False, ep_ret=ep[0], fin_stats=ep[1])
+                act = acts[p] if acts is not None else wo.gen_actions(self.gen, st["steps"], self.body.n_muscle)
+                out = wo.step(self.body, prm, st, act, want_info=False, ep_ret=ep[0], fin_stats=ep[1])
                 self.parts[p] = (a, b, prm, st, ep, out["obs"])
                 self.nonfinite += int((~np.isfinite(out["obs"]).all(1)).sum())
                 self.done_count += int(out["done"].sum())
+                if split["obs"] is not None:
+                    self._count_obs(out["obs"])
                 for k, want in (("obs", out["obs"]), ("reward", out["reward"]), ("done", out["done"].astype(bool))):
                     if split[k] is not None:
                         g = split[k][p].astype(bool) if k == "done" else split[k][p]
@@ -284,28 +302,66 @@ def seven_size(which):
     return {"2^17": 1 << 17, "6*SMs*128+1": 6 * sms * 128 + 1, "7*SMs*128": 7 * sms * 128, "6*SMs*128": 6 * sms * 128}[which]
 
 
+_PROBE_BUILDERS = {}
+_PROFILED = []
+
+
+def register_probes(builder):
+    """Adds builder() -> [(probe label, run)] to the one profiler session of this process (see kernel_names)."""
+    _PROBE_BUILDERS[f"{builder.__module__}.{builder.__name__}"] = builder
+    return builder
+
+
+def kernel_names():
+    """{probe label: name of the step or package-physics kernel that the probe's run launched}, or None when
+    torch.profiler reports no kernel names.  One profiler session for the probes of every test module loaded in this
+    process, on first use: a second session in the same process may see no device activity.  Every probe's objects
+    are built before the session and each run launches exactly one such kernel, so the kernels are told apart by their
+    launch order."""
+    if _PROFILED:
+        return _PROFILED[0]
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    probes = [p for build in _PROBE_BUILDERS.values() for p in build()]
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _, run in probes:
+            run()
+            torch.cuda.synchronize()
+    ev = sorted((e for e in prof.events() if re.search(r"step_\w*kernel|pkg_update\w*kernel", e.name)),
+                key=lambda e: e.time_range.start)
+    names = None
+    if ev:
+        assert len(ev) == len(probes), [e.name for e in ev]
+        names = {label: e.name for (label, _), e in zip(probes, ev)}
+    _PROFILED.append(names)
+    return names
+
+
+@register_probes
+def _seven_cta_probes():
+    import torch
+    out = []
+    for w in SEVEN_SIZES:
+        e = _env(seven_size(w), graph_safe=True)
+        a = torch.zeros(e.num_envs, e.M, device=DEV)
+        out.append((f"step {w}", lambda e=e, a=a: e.step(a)))
+    return out
+
+
 @pytest.fixture(scope="module")
 def step_kernel_minb():
     """{size id: MINB template argument of the step kernel one step at that size launched (0 = default)}, or None when
-    torch.profiler reports no kernel names.  One profiler session for all sizes: a second session in the same process
-    may see no device activity, so the kernels are told apart by their launch order."""
-    import torch
-    from torch.profiler import ProfilerActivity, profile
-    envs = [_env(seven_size(w), graph_safe=True) for w in SEVEN_SIZES]
-    acts = [torch.zeros(e.num_envs, e.M, device=DEV) for e in envs]
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        for e, a in zip(envs, acts):
-            e.step(a)
-            torch.cuda.synchronize()
-    ev = sorted((e for e in prof.events() if "step_static_packed_kernel" in e.name), key=lambda e: e.time_range.start)
-    if not ev:
+    torch.profiler reports no kernel names."""
+    names = kernel_names()
+    if names is None:
         return None
-    assert len(ev) == len(SEVEN_SIZES), [e.name for e in ev]
     out = {}
-    for w, e in zip(SEVEN_SIZES, ev):  # demangled "...StepArgs<4, 5>, 7>(...)" (or "(int)7"), or mangled "...ELi7EEEvT3_"
-        m = re.search(r"step_static_packed_kernel<.*,\s*(?:\(int\))?(\d+)\s*>\s*\(", e.name) or re.search(r"Li(\d+)EEEvT", e.name)
-        out[w] = int(m.group(1)) if m else e.name
+    for w in SEVEN_SIZES:   # demangled "...StepArgs<4, 5>, 7>(...)" (or "(int)7"), or mangled "...ELi7EEEvT3_"
+        name = names[f"step {w}"]
+        assert "step_static_packed_kernel" in name, (w, name)
+        m = re.search(r"step_static_packed_kernel<.*,\s*(?:\(int\))?(\d+)\s*>\s*\(", name) or re.search(r"Li(\d+)EEEvT", name)
+        out[w] = int(m.group(1)) if m else name
     return out
 
 
