@@ -17,7 +17,7 @@
  *   action          : row-major [E][act_dim] (act_layout 0) or feature-major [act_dim][E] (act_layout 1)
  *   obs             : row-major [E][D] (obs_layout 0) or feature-major [D][E] (obs_layout 1)
  *   reward [E], done uint8 [E], contact_* uint32 bitmask [E] (bit n = mass n)
- *   energy [E], centroid [3][E], ep_ret [E], fin_stats [4][E]
+ *   energy [E], centroid [3][E], ep_ret [E], fin_stats [4][E], nf_stats [2][E]
  *   noise           : SoA like pos; already scaled by sigma
  * D = 3 * (in3d ? 3 : 2) * n_mass + n_muscle   (Creature.getstat, gym/optimized_walker.py:129-162)
  *
@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define WG_ABI_VERSION 3
+#define WG_ABI_VERSION 4
 #define WG_MAX_MASS 32
 #define WG_MAX_SPRING 96
 
@@ -93,6 +93,11 @@ typedef struct wg_params {
     uint32_t seed_lo, seed_hi;   /* Philox key of the in-kernel jitter */
     uint32_t step_index;    /* global step number (Philox counter word), set by the caller each step */
     uint32_t env_offset;    /* global id of env 0 of this shard (multi-GPU invariance) */
+    int32_t  end_nonfinite; /* 0 = the reference's done rule; 1 = also done on a step whose reward is not finite
+                               (!(|reward| <= FLT_MAX)): an env whose state overflowed to inf / NaN ends its episode and,
+                               with auto_reset 2, restarts from the template.  Needs auto_reset 0 or 2 (a jitter reset
+                               keeps the overflowed positions) */
+    int32_t  reserved1;
 } wg_params;
 
 /*
@@ -155,6 +160,9 @@ typedef struct wg_buffers {
     /* wg_step_multi only: HOST pointer to an in-kernel action source (copied into the kernel parameters at launch);
      * when set with mode != 0, action must be NULL and n_action_steps is ignored */
     const wg_action_gen* action_gen;
+    float*       nf_stats;      /* in/out, optional: per-env sums over finished episodes whose return is not finite:
+                                   [0] count, [1] length.  Such an episode then goes here instead of into fin_stats.
+                                   Needs fin_stats and the running return (ep_ret, or state_packed) */
 } wg_buffers;
 
 /*
@@ -294,9 +302,12 @@ int wg_reset(const wg_topology* topo, const wg_params* prm, const wg_buffers* bu
 
 /*
  * Sum the per-env finished-episode accumulators into out8 (device, 8 doubles):
- * [sum return, sum return^2, sum length, count, 0, 0, 0, 0].  The caller
+ * [sum return, sum return^2, sum length, count, non-finite count, non-finite length, 0, 0].
+ * nf_stats may be NULL (then out8[4..5] = 0).  One kernel launch.  The caller
  * all-reduces out8 across ranks (NCCL) -- the only collective on this path.
+ * wg_stats_reduce(f, n, o, s) is wg_stats_reduce_split(f, NULL, n, o, s).
  */
+int wg_stats_reduce_split(const float* fin_stats, const float* nf_stats, int64_t n_env, double* out8, void* cuda_stream);
 int wg_stats_reduce(const float* fin_stats, int64_t n_env, double* out8, void* cuda_stream);
 
 /*

@@ -10,7 +10,7 @@ import ctypes as C
 import os
 
 MAX_MASS, MAX_SPRING = 32, 96
-ABI_VERSION = 3
+ABI_VERSION = 4
 GEN_MAX_ROWS, GEN_MAX_MUSCLE = 32, 16
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -41,6 +41,7 @@ class WgParams(C.Structure):
         ("in3d", C.c_int32), ("max_steps", C.c_int32), ("k_sub", C.c_int32), ("auto_reset", C.c_int32),
         ("integrator", C.c_int32),
         ("seed_lo", C.c_uint32), ("seed_hi", C.c_uint32), ("step_index", C.c_uint32), ("env_offset", C.c_uint32),
+        ("end_nonfinite", C.c_int32), ("reserved1", C.c_int32),          # 1 = a non-finite reward ends the episode
     ]
 
 
@@ -64,6 +65,7 @@ class WgBuffers(C.Structure):
         ("step_counter", C.c_void_p), ("state_packed", C.c_void_p),
         ("mx64", C.c_void_p), ("mx_weak", C.c_void_p), ("action64", C.c_void_p),      # x64 mode (wg_step_x64)
         ("action_gen", C.POINTER(WgActionGen)),                                         # wg_step_multi: in-kernel action source
+        ("nf_stats", C.c_void_p),                                                       # [2][E] non-finite episodes
     ]
 
 
@@ -100,7 +102,7 @@ TUNE_TMA, TUNE_PART, TUNE_L2_PREFETCH, TUNE_JIT, TUNE_POLICY_TC, TUNE_PDL = 0, 1
 
 EXPORTS = ("wg_abi_version", "wg_last_error_string", "wg_obs_dim", "wg_kernel_variant", "wg_force_generic",
            "wg_set_tuning", "wg_packed_state_floats", "wg_packed_available", "wg_jit_prepare",
-           "wg_step", "wg_step_multi", "wg_step_x64", "wg_reset", "wg_stats_reduce", "wg_step_host", "wg_step_multi_host", "wg_pkg_update_physics", "wg_pkg_kernel_variant",
+           "wg_step", "wg_step_multi", "wg_step_x64", "wg_reset", "wg_stats_reduce", "wg_stats_reduce_split", "wg_step_host", "wg_step_multi_host", "wg_pkg_update_physics", "wg_pkg_kernel_variant",
            "wg_policy_act", "wg_policy_step", "wg_gae", "wg_stream_probe", "wg_host_alloc", "wg_host_free", "wg_getstat", "wg_policy_tc_status",
            "wg_selftest_div_smallint", "wg_selftest_forced_list", "wg_selftest_sqrt", "wg_selftest_div3")
 
@@ -150,6 +152,7 @@ def load():
     lib.wg_step_x64.restype = C.c_int
     lib.wg_reset.argtypes = [P(WgTopology), P(WgParams), P(WgBuffers), C.c_int64, C.c_int, C.c_void_p, C.c_void_p]
     lib.wg_stats_reduce.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
+    lib.wg_stats_reduce_split.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
     lib.wg_step_host.argtypes = [P(WgTopology), P(WgParams), P(WgBuffers), C.c_int64,
                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.wg_pkg_update_physics.argtypes = [P(WgPkgSystem), P(WgPkgParams), C.c_void_p, C.c_void_p, C.c_void_p,
@@ -180,7 +183,7 @@ def load():
                  "wg_selftest_sqrt", "wg_selftest_div3"):
         getattr(lib, name).restype = C.c_int
     for name in ("wg_obs_dim", "wg_kernel_variant", "wg_force_generic", "wg_step", "wg_reset",
-                 "wg_stats_reduce", "wg_step_host", "wg_pkg_update_physics", "wg_policy_act", "wg_gae"):
+                 "wg_stats_reduce", "wg_stats_reduce_split", "wg_step_host", "wg_pkg_update_physics", "wg_policy_act", "wg_gae"):
         getattr(lib, name).restype = C.c_int
     _lib = lib
     return lib

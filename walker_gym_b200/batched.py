@@ -26,6 +26,7 @@ from .topology import topology_from_creature
 from .walker import Creature, create_balance_creature, create_box_creature, make_creature, BODIES
 
 AUTO_RESET = {None: 0, False: 0, "none": 0, "jitter": 1, "reference": 1, "template": 2, True: 2}
+NONFINITE = ("keep", "count", "end")
 
 
 def creature_from_id(env_id: str) -> Creature:
@@ -43,9 +44,10 @@ def creature_from_id(env_id: str) -> Creature:
 
 def make_params(*, in3d=False, g=100, dampk=0, ground_high=0, ground_k=1000, ground_damp=100, friction=100,
                 rand_sigma=0.1, time_step=0.01, max_steps=1000, k_sub=1, auto_reset=0, seed=0,
-                step_index=0, env_offset=0, integrator="run1") -> WgParams:
+                step_index=0, env_offset=0, integrator="run1", end_nonfinite=False) -> WgParams:
     """PhysicsEnv's constructor arguments -> ``wg_params``.  Scalars are converted
-    the way NumPy converts the reference's python numbers at their point of use."""
+    the way NumPy converts the reference's python numbers at their point of use.
+    ``end_nonfinite``: a step whose reward is not finite also sets ``done`` (not in the reference)."""
     p = WgParams()
     p.g = float(g)
     p.dampk = np.float32(dampk)
@@ -60,6 +62,7 @@ def make_params(*, in3d=False, g=100, dampk=0, ground_high=0, ground_k=1000, gro
     p.in3d, p.max_steps, p.k_sub, p.auto_reset = int(bool(in3d)), int(max_steps), int(k_sub), int(auto_reset)
     p.seed_lo, p.seed_hi = int(seed) & 0xFFFFFFFF, (int(seed) >> 32) & 0xFFFFFFFF
     p.step_index, p.env_offset = int(step_index) & 0xFFFFFFFF, int(env_offset) & 0xFFFFFFFF
+    p.end_nonfinite = int(bool(end_nonfinite))
     return p
 
 
@@ -71,7 +74,25 @@ class BatchedPhysicsEnv:
                  env_offset: int = 0, graph_safe: bool = False, integrator: str = "run1",
                  state_layout: str = "auto", x64: bool = False,
                  track_info: bool = False, track_stats: bool = True, track_contacts: bool = False,
-                 keep_old_a: bool = False, initial_reset: bool = True):
+                 keep_old_a: bool = False, initial_reset: bool = True, nonfinite: str = "keep"):
+        """``nonfinite`` decides what happens to an env whose state overflowed to inf / NaN (Balance-v0 as written does
+        so a few dozen steps after a reset; such an env then steps NaN arithmetic until ``max_steps``):
+          "keep"  -- the reference's semantics: nothing special; its episode return enters the statistics (and makes
+                     their mean NaN);
+          "count" -- the same dynamics, observations, rewards and dones, bit for bit; a finished episode whose return
+                     is not finite is counted apart (``episode_stats()["nonfinite_episodes"]``) instead of entering the
+                     return statistics;
+          "end"   -- as "count", and a step whose reward is not finite also sets ``done``, so the template auto-reset
+                     (or the caller, with ``auto_reset="none"``) restarts the env.  Not with ``auto_reset="jitter"``:
+                     a jitter reset keeps the overflowed positions."""
+        if nonfinite not in NONFINITE:
+            raise ValueError(f"nonfinite must be one of {NONFINITE}")
+        if nonfinite != "keep" and not track_stats:
+            raise ValueError(f"nonfinite={nonfinite!r} needs track_stats=True (it splits the episode statistics)")
+        if nonfinite == "end" and AUTO_RESET.get(auto_reset) == 1:
+            raise ValueError("nonfinite='end' needs auto_reset='template' or 'none': a jitter reset keeps the "
+                             "overflowed positions and cannot bring the env back")
+        self.nonfinite = nonfinite
         self.lib = _lib.load()
         self.device = torch.device(device)
         if self.device.type != "cuda":
@@ -93,7 +114,7 @@ class BatchedPhysicsEnv:
                                   ground_damp=ground_damp, friction=friction, rand_sigma=rand_sigma,
                                   time_step=time_step, max_steps=max_steps, k_sub=k_sub,
                                   auto_reset=AUTO_RESET[auto_reset], seed=seed, env_offset=env_offset,
-                                  integrator=integrator)
+                                  integrator=integrator, end_nonfinite=nonfinite == "end")
         self.N, self.M = self.topo.n_mass, self.topo.n_muscle
         self.obs_dim = self.lib.wg_obs_dim(C.byref(self.topo), int(self.in3d))
         self.obs_layout = obs_layout
@@ -150,6 +171,8 @@ class BatchedPhysicsEnv:
         self.contact_pre = torch.zeros(E, dtype=torch.int32, device=dev) if track_contacts else None
         self.contact_post = torch.zeros(E, dtype=torch.int32, device=dev) if track_contacts else None
         self.fin_stats = torch.zeros(4, E, dtype=f32, device=dev) if track_stats else None
+        # [0] count, [1] length sum of finished episodes whose return is not finite ("count" / "end" only)
+        self.nf_stats = torch.zeros(2, E, dtype=f32, device=dev) if nonfinite != "keep" else None
         self._stats_out = torch.zeros(8, dtype=torch.float64, device=dev)
         # graph_safe: the Philox step index lives in a device scalar advanced by a device op, so a
         # captured CUDA graph that replays step() keeps drawing fresh reset jitter
@@ -183,7 +206,7 @@ class BatchedPhysicsEnv:
         b.obs_layout = 0 if self.obs_layout == "row" else 1
         b.contact_pre, b.contact_post = self._p(self.contact_pre), self._p(self.contact_post)
         b.energy, b.centroid = self._p(self.energy), self._p(self.centroid)
-        b.ep_ret, b.fin_stats = self._p(self._ep_ret), self._p(self.fin_stats)
+        b.ep_ret, b.fin_stats, b.nf_stats = self._p(self._ep_ret), self._p(self.fin_stats), self._p(self.nf_stats)
         b.action, b.act_dim, b.noise = None, 0, None
         b.act_layout = 0 if self.act_layout == "row" else 1
         b.step_counter = self._p(self._counter)
@@ -570,17 +593,26 @@ class BatchedPhysicsEnv:
     def episode_stats(self, all_reduce: bool = False, clear: bool = False) -> dict:
         """Sum of finished-episode returns / squared returns / lengths / count over
         this shard; with ``all_reduce`` the 8-double vector is summed across ranks
-        (NCCL) -- the only collective anywhere near the step path."""
+        (NCCL) -- the only collective anywhere near the step path.  With ``nonfinite``
+        "count" / "end" the return statistics cover the finite episodes and the dict adds
+        ``nonfinite_episodes`` and ``nonfinite_length_mean``."""
         if self.fin_stats is None:
             raise RuntimeError("construct the env with track_stats=True")
         with torch.cuda.device(self.device):
-            rc = self.lib.wg_stats_reduce(self.fin_stats.data_ptr(), self.num_envs, self._stats_out.data_ptr(), self._stream())
+            if self.nf_stats is None:
+                rc = self.lib.wg_stats_reduce(self.fin_stats.data_ptr(), self.num_envs, self._stats_out.data_ptr(),
+                                              self._stream())
+            else:
+                rc = self.lib.wg_stats_reduce_split(self.fin_stats.data_ptr(), self.nf_stats.data_ptr(), self.num_envs,
+                                                    self._stats_out.data_ptr(), self._stream())
         _lib.check(rc, "wg_stats_reduce")
         from .dist import all_reduce_stats, finalize_stats
         out = all_reduce_stats(self._stats_out) if all_reduce else self._stats_out
-        stats = finalize_stats(out)
+        stats = finalize_stats(out, nonfinite=self.nf_stats is not None)
         if clear:
             self.fin_stats.zero_()
+            if self.nf_stats is not None:
+                self.nf_stats.zero_()
         return stats
 
     # ---- checkpoint / state.pkl ------------------------------------------------------
@@ -593,7 +625,7 @@ class BatchedPhysicsEnv:
              "obs": snap(self.obs), "step_count": self.step_count}
         if self.ep_ret is not None:
             d["ep_ret"] = snap(self.ep_ret)
-        for k in ("old_a", "fin_stats", "mx64", "mx_weak"):
+        for k in ("old_a", "fin_stats", "nf_stats", "mx64", "mx_weak"):
             if getattr(self, k) is not None:
                 d[k] = snap(getattr(self, k))
         if self._counter is not None:
@@ -609,7 +641,7 @@ class BatchedPhysicsEnv:
                 if self._counter is None:
                     raise ValueError("the checkpoint comes from a graph_safe env (device step counter); this env has none")
                 self._counter.copy_(torch.as_tensor(v, device=self.device).reshape(1))
-            elif k in ("obs", "old_a", "fin_stats", "mx64", "mx_weak") and getattr(self, k, None) is not None:
+            elif k in ("obs", "old_a", "fin_stats", "nf_stats", "mx64", "mx_weak") and getattr(self, k, None) is not None:
                 getattr(self, k).copy_(v)       # after set_state: the saved float64 muscle state wins over its float32 view
 
     def save_state(self, path: str, env_index: int = 0) -> None:

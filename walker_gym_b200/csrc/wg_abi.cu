@@ -105,6 +105,11 @@ static int validate(const wg_topology* t, const wg_params* p, const wg_buffers* 
     if (p->k_sub < 1) return fail(WG_ERR_BAD_ARG, "k_sub must be >= 1%s");
     if (p->auto_reset < 0 || p->auto_reset > 2) return fail(WG_ERR_BAD_ARG, "auto_reset must be 0, 1 or 2%s");
     if (p->integrator < 0 || p->integrator > 1) return fail(WG_ERR_BAD_ARG, "integrator must be 0 (run1) or 1 (run2)%s");
+    if (p->end_nonfinite != 0 && p->end_nonfinite != 1) return fail(WG_ERR_BAD_ARG, "end_nonfinite must be 0 or 1%s");
+    if (p->end_nonfinite && p->auto_reset == 1)
+        return fail(WG_ERR_BAD_ARG, "end_nonfinite needs auto_reset 0 or 2: a jitter reset keeps the overflowed positions%s");
+    if (b->nf_stats && (!b->fin_stats || (!b->ep_ret && !b->state_packed)))
+        return fail(WG_ERR_BAD_ARG, "nf_stats needs fin_stats and the running return (ep_ret or state_packed)%s");
     if (b->state_packed) {
         if (!packed_pick(t))
             return fail(WG_ERR_BAD_ARG, "the packed state layout needs a body with wg_packed_available() == 1%s");
@@ -286,9 +291,13 @@ int wg_reset(const wg_topology* topo, const wg_params* prm, const wg_buffers* bu
     return launch_reset(topo, prm, buf, n_env, mode, mask, (cudaStream_t)cuda_stream);
 }
 
-int wg_stats_reduce(const float* fin_stats, int64_t n_env, double* out8, void* cuda_stream) {
+int wg_stats_reduce_split(const float* fin_stats, const float* nf_stats, int64_t n_env, double* out8, void* cuda_stream) {
     if (!fin_stats || !out8 || n_env < 0) return fail(WG_ERR_BAD_ARG, "bad argument to wg_stats_reduce%s");
-    return launch_stats(fin_stats, n_env, out8, (cudaStream_t)cuda_stream);
+    return launch_stats(fin_stats, nf_stats, n_env, out8, (cudaStream_t)cuda_stream);
+}
+
+int wg_stats_reduce(const float* fin_stats, int64_t n_env, double* out8, void* cuda_stream) {
+    return wg_stats_reduce_split(fin_stats, nullptr, n_env, out8, cuda_stream);
 }
 
 int wg_step_host(const wg_topology* topo, const wg_params* prm, const wg_buffers* buf, int64_t n_env,

@@ -152,8 +152,8 @@ int launch_reset(const wg_topology* t, const wg_params* p, const wg_buffers* b, 
     return WG_OK;
 }
 
-int launch_stats(const float* fin_stats, int64_t E, double* out8, cudaStream_t s) {
-    stats_reduce_kernel<1024><<<1, 1024, 0, s>>>(fin_stats, E, out8);
+int launch_stats(const float* fin_stats, const float* nf_stats, int64_t E, double* out8, cudaStream_t s) {
+    stats_reduce_kernel<1024><<<1, 1024, 0, s>>>(fin_stats, nf_stats, E, out8);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail(WG_ERR_CUDA, "stats kernel launch: %s", cudaGetErrorString(e));
     return WG_OK;

@@ -34,7 +34,12 @@ struct StepArgs {
     int64_t E;
     int32_t pf_dist;          // packed kernel: L2 prefetch distance in tiles (0 = off)
     int32_t act_dim, act_layout;
+    float* nf_stats;          // optional [2][E]: count and length sum of finished episodes whose return is not finite
 };
+
+// NF (template flag of the kernel families whose keep-mode code must stay exactly what it was, see
+// step_static_packed_kernel): false compiles the non-finite handling out -- the instance then ignores
+// ec.end_nonfinite and nf_stats, and the host launches it only when both are off.
 
 // ---- TMA 1-D bulk store helpers (shared memory -> global), used for the observation rows ----------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -86,7 +91,7 @@ __device__ __forceinline__ void st_vec(T* p, const T (&in)[EPT]) {
 struct EpiOut { float reward; uint32_t cpost; int done; float energy; float cen[3]; };
 
 // reward, done and info from the per-mass heights ys(i) and speeds sp(i) (already filled in)
-template <class BV, class Store, class YS, class SP>
+template <bool NF = true, class BV, class Store, class YS, class SP>
 __device__ __forceinline__ void epilogue_reduce(int N, const BV& bv, const EnvConst& ec, Store& st, int32_t steps_now,
                                                 bool want_energy, bool want_centroid, YS ys, SP sp, EpiOut& o) {
     uint32_t cpost = 0; int ncon = 0;
@@ -109,6 +114,9 @@ __device__ __forceinline__ void epilogue_reduce(int N, const BV& bv, const EnvCo
         for (int n = 0; n < N; n++) all_stopped = all_stopped && (sp(n) < 0.1f);
         if (all_stopped && steps_now > 100) dn = 1;
     }
+    // opt-in (wg_params.end_nonfinite): an env whose state overflowed ends its episode.  The reward sums every mass
+    // height and speed, so an inf / NaN anywhere in the state reaches it in the same step.
+    if (NF && ec.end_nonfinite && !is_finite(o.reward)) dn = 1;
     o.done = dn;
     if (want_energy) {                                           // _calculate_energy (:240-248)
         const float ke = np_pairwise_sum(N, [&](int i) { return bv.mass_f[i] * (sp(i) * sp(i)); });
@@ -126,7 +134,25 @@ __device__ __forceinline__ void epilogue_reduce(int N, const BV& bv, const EnvCo
     }
 }
 
-template <bool IN3D, class Topo, class BV, class Store, class YS, class SP>
+// episode statistics of env i whose episode just ended with return r after len steps: fin_stats [4][E] sums return,
+// return^2, length and count.  With nf_stats [2][E] bound, an episode whose return is not finite is counted there
+// instead (count, length sum), so one overflowed episode cannot make the mean return of the whole batch NaN.
+// Every step kernel accounts a finished episode through this function.
+template <bool NF = true, class Args>
+__device__ __forceinline__ void account_episode(const Args& A, int64_t E, int64_t i, float r, int32_t len) {
+    if (!A.fin_stats) return;
+    if (NF && A.nf_stats && !is_finite(r)) {
+        A.nf_stats[0 * E + i] += 1.0f;
+        A.nf_stats[1 * E + i] += (float)len;
+        return;
+    }
+    A.fin_stats[0 * E + i] += r;
+    A.fin_stats[1 * E + i] += r * r;
+    A.fin_stats[2 * E + i] += (float)len;
+    A.fin_stats[3 * E + i] += 1.0f;
+}
+
+template <bool IN3D, bool NF = true, class Topo, class BV, class Store, class YS, class SP>
 __device__ __forceinline__ void epilogue(const Topo& topo, const BV& bv, const EnvConst& ec, Store& st,
                                          int32_t steps_now, bool want_energy, bool want_centroid,
                                          YS ys, SP sp, EpiOut& o) {
@@ -136,7 +162,7 @@ __device__ __forceinline__ void epilogue(const Topo& topo, const BV& bv, const E
         ys(n) = st.pos(n, 1);
         sp(n) = np_norm3(v3(st.vel(n, 0), st.vel(n, 1), st.vel(n, 2)));
     }
-    epilogue_reduce(N, bv, ec, st, steps_now, want_energy, want_centroid, ys, sp, o);
+    epilogue_reduce<NF>(N, bv, ec, st, steps_now, want_energy, want_centroid, ys, sp, o);
 }
 
 // =================================================================================
@@ -250,12 +276,7 @@ step_static_kernel(const __grid_constant__ Args A) {
             stp[j] = sn;
             if (A.ep_ret) {
                 const float r = epr[j] + o.reward;
-                if (o.done && A.fin_stats) {
-                    A.fin_stats[0 * E + e + j] += r;
-                    A.fin_stats[1 * E + e + j] += r * r;
-                    A.fin_stats[2 * E + e + j] += (float)sn;
-                    A.fin_stats[3 * E + e + j] += 1.0f;
-                }
+                if (o.done) account_episode(A, E, e + j, r, sn);
                 epr[j] = (o.done && A.ec.auto_reset) ? 0.0f : r;
             }
             if (o.done && A.ec.auto_reset) {
@@ -456,12 +477,7 @@ step_generic_kernel(const __grid_constant__ StepArgs<kMaxMass, kMaxSpring> A, co
         if (A.centroid) { A.centroid[e] = o.cen[0]; A.centroid[E + e] = o.cen[1]; A.centroid[2 * E + e] = o.cen[2]; }
         if (A.ep_ret) {
             const float r = A.ep_ret[e] + o.reward;
-            if (o.done && A.fin_stats) {
-                A.fin_stats[0 * E + e] += r;
-                A.fin_stats[1 * E + e] += r * r;
-                A.fin_stats[2 * E + e] += (float)sn;
-                A.fin_stats[3 * E + e] += 1.0f;
-            }
+            if (o.done) account_episode(A, E, e, r, sn);
             A.ep_ret[e] = (o.done && A.ec.auto_reset) ? 0.0f : r;
         }
         if (o.done && A.ec.auto_reset) {
@@ -585,19 +601,26 @@ reset_kernel(const __grid_constant__ StepArgs<kMaxMass, kMaxSpring> A, int mode,
 }
 
 // =================================================================================
-// K3: deterministic single-block reduction of the finished-episode accumulators.
+// K3: deterministic single-block reduction of the finished-episode accumulators:
+// out8 = [fin_stats rows 0..3, nf_stats rows 0..1 (0 when nf is null), 0, 0].
 // =================================================================================
 template <int THREADS>
-__global__ void __launch_bounds__(THREADS) stats_reduce_kernel(const float* __restrict__ fin, int64_t E, double* out8) {
-    __shared__ double part[4][32];
-    double acc[4] = { 0.0, 0.0, 0.0, 0.0 };
+__global__ void __launch_bounds__(THREADS) stats_reduce_kernel(const float* __restrict__ fin, const float* __restrict__ nf,
+                                                               int64_t E, double* out8) {
+    constexpr int Q = 6;
+    __shared__ double part[Q][32];
+    double acc[Q] = { 0.0, 0.0, 0.0, 0.0, 0.0, 0.0 };
     for (int64_t i = threadIdx.x; i < E; i += blockDim.x) {
 #pragma unroll
         for (int q = 0; q < 4; q++) acc[q] += (double)fin[(int64_t)q * E + i];
+        if (nf) {
+            acc[4] += (double)nf[i];
+            acc[5] += (double)nf[E + i];
+        }
     }
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
-    for (int q = 0; q < 4; q++) {
+    for (int q = 0; q < Q; q++) {
 #pragma unroll
         for (int off = 16; off > 0; off >>= 1) acc[q] += __shfl_down_sync(0xffffffffu, acc[q], off);
         if (lane == 0) part[q][warp] = acc[q];
@@ -605,12 +628,13 @@ __global__ void __launch_bounds__(THREADS) stats_reduce_kernel(const float* __re
     __syncthreads();
     if (warp == 0) {
 #pragma unroll
-        for (int q = 0; q < 4; q++) {
+        for (int q = 0; q < Q; q++) {
             double v = lane < (int)(blockDim.x >> 5) ? part[q][lane] : 0.0;
 #pragma unroll
             for (int off = 16; off > 0; off >>= 1) v += __shfl_down_sync(0xffffffffu, v, off);
-            if (lane == 0) { out8[q] = v; out8[4 + q] = 0.0; }
+            if (lane == 0) out8[q] = v;
         }
+        if (lane == 0) { out8[6] = 0.0; out8[7] = 0.0; }
     }
 }
 

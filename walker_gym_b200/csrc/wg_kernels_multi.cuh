@@ -57,7 +57,8 @@ __device__ __forceinline__ float gen_action(const ActionGen& G, int m, int32_t s
 // last step.
 // GEN: compile-time switch for the in-kernel action sources -- the tensor-action instance (GEN = false) stays exactly
 // the code it was (the loop is instruction-cache sensitive: a run-time branch around the generator cost it 6 %).
-template <class Topo, bool IN3D, int MM, class Args = StepArgs<Topo::N, Topo::S>, bool GEN = false>
+// NF: as for step_static_packed_kernel (the non-finite handling compiled in; launched with it off only as NF = false).
+template <class Topo, bool IN3D, int MM, class Args = StepArgs<Topo::N, Topo::S>, bool GEN = false, bool NF = true>
 __global__ void __launch_bounds__(kMultiBlock, multi_min_blocks(Topo::N))
 step_multi_packed_kernel(const __grid_constant__ Args A, const int n_steps, const int64_t act_stride,
                          const __grid_constant__ ActionGen G) {
@@ -134,17 +135,12 @@ step_multi_packed_kernel(const __grid_constant__ Args A, const int n_steps, cons
             const int32_t sn = stp + 1;
             float ysr[N], spr[N];
             EpiOut o;
-            epilogue<IN3D>(topo, A.bv, A.ec, st, sn, false, false,
+            epilogue<IN3D, NF>(topo, A.bv, A.ec, st, sn, false, false,
                            [&](int i) -> float& { return ysr[i]; }, [&](int i) -> float& { return spr[i]; }, o);
             stp = sn;
             {
                 const float r = epr + o.reward;
-                if (o.done && A.fin_stats) {
-                    A.fin_stats[0 * E + e] += r;
-                    A.fin_stats[1 * E + e] += r * r;
-                    A.fin_stats[2 * E + e] += (float)sn;
-                    A.fin_stats[3 * E + e] += 1.0f;
-                }
+                if (o.done) account_episode<NF>(A, E, e, r, sn);
                 epr = (o.done && A.ec.auto_reset) ? 0.0f : r;
             }
             if (o.done && A.ec.auto_reset) {
@@ -210,8 +206,10 @@ inline int launch_multi_packed(const wg_topology* t, const wg_params* p, const w
     const size_t smem = b->obs ? sizeof(float) * kMultiBlock * (bulk ? D : (D | 1)) : 0;
     static thread_local ActionGen G;
     fill_gen(G, b);
-    auto kern = G.mode ? step_multi_packed_kernel<Topo, IN3D, MM, StepArgs<Topo::N, Topo::S>, true>
-                       : step_multi_packed_kernel<Topo, IN3D, MM, StepArgs<Topo::N, Topo::S>, false>;
+    using SA = StepArgs<Topo::N, Topo::S>;
+    const bool nf = p->end_nonfinite || b->nf_stats;
+    auto kern = G.mode ? (nf ? step_multi_packed_kernel<Topo, IN3D, MM, SA, true, true> : step_multi_packed_kernel<Topo, IN3D, MM, SA, true, false>)
+                       : (nf ? step_multi_packed_kernel<Topo, IN3D, MM, SA, false, true> : step_multi_packed_kernel<Topo, IN3D, MM, SA, false, false>);
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return fail(WG_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));

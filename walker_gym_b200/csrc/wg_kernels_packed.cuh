@@ -23,13 +23,15 @@ static_assert(kPackedBlock % 128 == 0, "the packed layout is tiled by 128 envs")
 
 // Args: StepArgs<Topo::N, Topo::S> for the ahead-of-time specialisations; the run-time compiled ones (wg_jit.cu) take
 // the full-size StepArgs<kMaxMass, kMaxSpring> the host can fill for any body.
+// NF: the non-finite handling (wg_params.end_nonfinite, buf->nf_stats) is compiled in; the launcher takes the NF = false
+// instance when both are off, so the reference's semantics run exactly the code they ran before the option existed.
 // MINB: resident CTAs per SM the compiler must allow (0 = the default for the body size).  The 7-CTA instance (72
 // registers) exists for grids that fit ONE wave at 7 CTAs per SM but not at 6 -- BASELINE config 3 as written, 2^20 envs
 // over 8 GPUs = 1024 CTAs per GPU against 148 x 6 = 888 slots: a second, 14 %-full wave would double the step time.
 __host__ __device__ constexpr int packed_min_blocks(int n_mass, int minb) {
     return minb > 0 ? minb : (n_mass <= 4 ? WG_PACKED_MIN_BLOCKS : (n_mass <= 6 ? 512 : 384) / WG_PACKED_BLOCK);
 }
-template <class Topo, bool IN3D, int OBS, int MM, class Args = StepArgs<Topo::N, Topo::S>, int MINB = 0>
+template <class Topo, bool IN3D, int OBS, int MM, class Args = StepArgs<Topo::N, Topo::S>, bool NF = true, int MINB = 0>
 __global__ void __launch_bounds__(kPackedBlock, packed_min_blocks(Topo::N, MINB))
 step_static_packed_kernel(const __grid_constant__ Args A) {
     constexpr int N = Topo::N, M = Topo::M;
@@ -110,17 +112,12 @@ step_static_packed_kernel(const __grid_constant__ Args A) {
         const int32_t sn = stp + 1;
         float ysr[N], spr[N];
         EpiOut o;
-        epilogue<IN3D>(topo, A.bv, A.ec, st, sn, A.energy != nullptr, A.centroid != nullptr,
+        epilogue<IN3D, NF>(topo, A.bv, A.ec, st, sn, A.energy != nullptr, A.centroid != nullptr,
                        [&](int i) -> float& { return ysr[i]; }, [&](int i) -> float& { return spr[i]; }, o);
         stp = sn;
         {   // episode statistics: the running return lives in the packed state
             const float r = epr + o.reward;
-            if (o.done && A.fin_stats) {
-                A.fin_stats[0 * E + e] += r;
-                A.fin_stats[1 * E + e] += r * r;
-                A.fin_stats[2 * E + e] += (float)sn;
-                A.fin_stats[3 * E + e] += 1.0f;
-            }
+            if (o.done) account_episode<NF>(A, E, e, r, sn);
             epr = (o.done && A.ec.auto_reset) ? 0.0f : r;
         }
         if (o.done && A.ec.auto_reset) {

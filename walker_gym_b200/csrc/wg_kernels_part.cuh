@@ -165,12 +165,7 @@ step_part_kernel(const __grid_constant__ PartArgs PA) {
         if (A.centroid) { A.centroid[e] = o.cen[0]; A.centroid[E + e] = o.cen[1]; A.centroid[2 * E + e] = o.cen[2]; }
         if (A.ep_ret) {
             const float r = A.ep_ret[e] + o.reward;
-            if (o.done && A.fin_stats) {
-                A.fin_stats[0 * E + e] += r;
-                A.fin_stats[1 * E + e] += r * r;
-                A.fin_stats[2 * E + e] += (float)sn;
-                A.fin_stats[3 * E + e] += 1.0f;
-            }
+            if (o.done) account_episode(A, E, e, r, sn);
             A.ep_ret[e] = (o.done && A.ec.auto_reset) ? 0.0f : r;
         }
         do_reset = (o.done && A.ec.auto_reset) ? 1 : 0;
@@ -398,12 +393,7 @@ step_units_kernel(const __grid_constant__ UnitsArgs<U, MM> UA) {
         if (A.centroid) { A.centroid[e] = o.cen[0]; A.centroid[E + e] = o.cen[1]; A.centroid[2 * E + e] = o.cen[2]; }
         if (A.ep_ret) {
             const float r = A.ep_ret[e] + o.reward;
-            if (o.done && A.fin_stats) {
-                A.fin_stats[0 * E + e] += r;
-                A.fin_stats[1 * E + e] += r * r;
-                A.fin_stats[2 * E + e] += (float)sn;
-                A.fin_stats[3 * E + e] += 1.0f;
-            }
+            if (o.done) account_episode(A, E, e, r, sn);
             A.ep_ret[e] = (o.done && A.ec.auto_reset) ? 0.0f : r;
         }
         do_reset = (o.done && A.ec.auto_reset) ? 1 : 0;

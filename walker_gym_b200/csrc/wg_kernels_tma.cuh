@@ -88,12 +88,7 @@ __device__ __forceinline__ void env_compute_store(const Args& A, RegStore<Topo::
             stp = sn;
             if (A.ep_ret) {
                 const float r = epr + o.reward;
-                if (o.done && A.fin_stats) {
-                    A.fin_stats[0 * E + e] += r;
-                    A.fin_stats[1 * E + e] += r * r;
-                    A.fin_stats[2 * E + e] += (float)sn;
-                    A.fin_stats[3 * E + e] += 1.0f;
-                }
+                if (o.done) account_episode(A, E, e, r, sn);
                 A.ep_ret[e] = (o.done && A.ec.auto_reset) ? 0.0f : r;
             }
             if (o.done && A.ec.auto_reset) {

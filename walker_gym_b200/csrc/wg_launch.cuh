@@ -66,7 +66,7 @@ int launch_insect(const wg_topology*, const wg_params*, const wg_buffers*, int64
 int launch_generic_step(const wg_topology*, const wg_params*, const wg_buffers*, int64_t E, cudaStream_t);
 int launch_part_step(const wg_topology*, const wg_params*, const wg_buffers*, int64_t E, int parts, cudaStream_t);
 int launch_reset(const wg_topology*, const wg_params*, const wg_buffers*, int64_t E, int mode, const uint8_t* mask, cudaStream_t);
-int launch_stats(const float* fin_stats, int64_t E, double* out8, cudaStream_t);
+int launch_stats(const float* fin_stats, const float* nf_stats, int64_t E, double* out8, cudaStream_t);
 
 // classify a host-known divisor for div_const (see wg_math.cuh)
 inline ConstDiv make_const_div(float m) {
@@ -115,6 +115,8 @@ inline void fill_args(StepArgs<MAXN, MAXS>& A, const wg_topology* t, const wg_pa
     ec.dt = p->dt; ec.dt2 = p->dt2; ec.sigma = p->sigma; ec.integrator = p->integrator;
     ec.max_steps = p->max_steps; ec.k_sub = p->k_sub; ec.auto_reset = p->auto_reset;
     ec.seed_lo = p->seed_lo; ec.seed_hi = p->seed_hi; ec.step_index = p->step_index; ec.env_offset = p->env_offset;
+    ec.end_nonfinite = p->end_nonfinite;
+    A.nf_stats = b->nf_stats;
     A.pos = b->pos; A.vel = b->vel; A.old_a = b->old_a; A.mx = b->mx; A.steps = b->steps;
     A.action = b->action; A.obs = b->obs; A.reward = b->reward; A.done = b->done;
     A.contact_pre = b->contact_pre; A.contact_post = b->contact_post; A.energy = b->energy; A.centroid = b->centroid;
@@ -213,12 +215,15 @@ inline int launch_static_packed(const wg_topology* t, const wg_params* p, const 
     constexpr int D = 3 * (IN3D ? 3 : 2) * Topo::N + Topo::M;
     constexpr bool bulk = (OBS == 1) && gcd_c(D, 32) <= 2;
     const size_t smem = (OBS == 1 && b->obs) ? sizeof(float) * kPackedBlock * (bulk ? D : (D | 1)) : 0;
-    auto kern = step_static_packed_kernel<Topo, IN3D, OBS, MM>;
+    using SA = StepArgs<Topo::N, Topo::S>;
+    const bool nf = p->end_nonfinite || b->nf_stats;          // the non-finite handling is compiled into NF = true only
+    auto kern = nf ? step_static_packed_kernel<Topo, IN3D, OBS, MM, SA, true> : step_static_packed_kernel<Topo, IN3D, OBS, MM, SA, false>;
     const int64_t n_blocks = (E + kPackedBlock - 1) / kPackedBlock;
     if constexpr (Topo::N <= 4 && IN3D && OBS == 1 && (MM == 0 || MM == 3) && WG_PACKED_MIN_BLOCKS == 6 && WG_PACKED_BLOCK == 128) {
         // a grid of (6, 7] CTAs per SM: one wave with the 7-CTA instance instead of one full wave plus a sliver
         const int64_t sms = sm_count();
-        if (n_blocks > 6 * sms && n_blocks <= 7 * sms) kern = step_static_packed_kernel<Topo, IN3D, OBS, MM, StepArgs<Topo::N, Topo::S>, 7>;
+        if (n_blocks > 6 * sms && n_blocks <= 7 * sms)
+            kern = nf ? step_static_packed_kernel<Topo, IN3D, OBS, MM, SA, true, 7> : step_static_packed_kernel<Topo, IN3D, OBS, MM, SA, false, 7>;
     }
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -44,6 +44,7 @@ struct EnvConst {
     int32_t max_steps, k_sub, auto_reset, integrator;
     uint32_t seed_lo, seed_hi, step_index, env_offset;
     int32_t dampk_is_zero;
+    int32_t end_nonfinite;  // 1 = a step whose reward is not finite ends the episode (epilogue_reduce)
 };
 
 // ---- state stores -------------------------------------------------------------

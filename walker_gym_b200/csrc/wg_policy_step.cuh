@@ -65,12 +65,7 @@ struct FusedStep {
         stp = sn;
         {   // episode statistics: the running return lives in the packed state
             const float r = epr + o.reward;
-            if (o.done && A.fin_stats) {
-                A.fin_stats[0 * E + e] += r;
-                A.fin_stats[1 * E + e] += r * r;
-                A.fin_stats[2 * E + e] += (float)sn;
-                A.fin_stats[3 * E + e] += 1.0f;
-            }
+            if (o.done) account_episode(A, E, e, r, sn);
             epr = (o.done && A.ec.auto_reset) ? 0.0f : r;
         }
         if (o.done && A.ec.auto_reset) {

@@ -34,25 +34,33 @@ def env_from_torchrun() -> Tuple[int, int, int]:
 
 
 def all_reduce_stats(vec: torch.Tensor) -> torch.Tensor:
-    """SUM all-reduce of the stats vector [return, return^2, length, count, 0, 0, 0, 0] (float64)."""
+    """SUM all-reduce of the stats vector [return, return^2, length, count, non-finite count, non-finite length, 0, 0]
+    (float64)."""
     if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
         vec = vec.clone()
         dist.all_reduce(vec, op=dist.ReduceOp.SUM)
     return vec
 
 
-def finalize_stats(vec) -> Dict[str, float]:
-    """Turn the (all-reduced) stats vector into mean / std / count."""
+def finalize_stats(vec, nonfinite: bool = False) -> Dict[str, float]:
+    """Turn the (all-reduced) stats vector into mean / std / count.  ``nonfinite``: the env counts episodes with a
+    non-finite return apart (``BatchedPhysicsEnv(nonfinite="count" | "end")``); the return statistics then cover the
+    finite episodes, and ``nonfinite_episodes`` / ``nonfinite_length_mean`` describe the others."""
     s = [float(x) for x in (vec.tolist() if hasattr(vec, "tolist") else vec)]
     n = s[3]
+    nan = float("nan")
     if n <= 0:
-        nan = float("nan")
-        return {"episodes": 0, "return_mean": nan, "return_std": nan, "length_mean": nan,
-                "return_sum": s[0], "return_sqsum": s[1], "length_sum": s[2]}
-    mean = s[0] / n
-    var = max(s[1] / n - mean * mean, 0.0)
-    return {"episodes": int(n), "return_mean": mean, "return_std": var ** 0.5, "length_mean": s[2] / n,
-            "return_sum": s[0], "return_sqsum": s[1], "length_sum": s[2]}
+        out = {"episodes": 0, "return_mean": nan, "return_std": nan, "length_mean": nan,
+               "return_sum": s[0], "return_sqsum": s[1], "length_sum": s[2]}
+    else:
+        mean = s[0] / n
+        var = max(s[1] / n - mean * mean, 0.0)
+        out = {"episodes": int(n), "return_mean": mean, "return_std": var ** 0.5, "length_mean": s[2] / n,
+               "return_sum": s[0], "return_sqsum": s[1], "length_sum": s[2]}
+    if nonfinite:
+        out["nonfinite_episodes"] = int(s[4])
+        out["nonfinite_length_mean"] = s[5] / s[4] if s[4] > 0 else nan
+    return out
 
 
 def make_sharded_env(creature, total_envs: int, *, device: Optional[torch.device] = None, **kwargs):
