@@ -67,8 +67,10 @@ typedef struct wg_topology {
     uint8_t sstring[WG_MAX_SPRING];     /* 1 = rope-type spring: no elastic force while shorter than its rest length
                                            (`if dx < 0 and string: f_size = 0`, Point.resilience,
                                            gym/optimized_engine.py:134-138, applied to Muscle.run / Skeleton.run; the
-                                           damping term is unchanged).  Bodies with such springs step through the
-                                           run-time-topology kernels. */
+                                           damping term is unchanged).  The rule holds for float32 and float64
+                                           (wg_step_x64) actions alike; with float64 actions a muscle's dx is the
+                                           double one.  Bodies with such springs step through the run-time-topology
+                                           kernels. */
 } wg_topology;
 
 /*
@@ -274,6 +276,10 @@ int wg_step_multi(const wg_topology* topo, const wg_params* prm, const wg_buffer
  * view of the lengths, which is what the float32 observation carries).  Bit-identical to the reference driven
  * with float64 actions.  Runs the run-time-topology kernel (a compatibility path, not the throughput path).
  * wg_reset does not touch mx64 / mx_weak: after a template reset the caller sets them to x0_d / 1.
+ * Returns WG_ERR_UNSUPPORTED for a body whose per-block tile (11 * n_mass + n_muscle + 3 rows of 129 floats) exceeds
+ * the device's shared memory per block (on a B200 with 32 masses: 93 or more muscles with row-major observations,
+ * 96 with feature-major ones); the check also runs when n_env == 0, so a call with no envs tells whether the body
+ * can step.
  */
 int wg_step_x64(const wg_topology* topo, const wg_x64* x64, const wg_params* prm, const wg_buffers* buf,
                 int64_t n_env, void* cuda_stream);

@@ -237,6 +237,7 @@ static void spring_run(const wgo_body *b, const wgo_params *p, env_state *s, int
         /* np.float64 length: dx, f_size and force in double; forced() adds force / m in double */
         double dx64 = (double)L - s->mx64[sp];
         double fs64 = (-dx64) * s->xb->sk_d[sp];
+        if (b->sstring[sp] && dx64 < 0) fs64 = 0.0;            /* rope-type, tested on the double dx */
         double F64[3], nF64[3];
         for (int c = 0; c < 3; c++) { F64[c] = fs64 * (double)dir[c]; nF64[c] = -F64[c]; }
         forced_list(s->acc[i], F64, b->mass[i], b->fixed[i]);

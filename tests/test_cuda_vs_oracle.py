@@ -342,9 +342,21 @@ def _random_spec(rng, N, S, M):
     return {"points": pts, "muscles": mus, "skeletons": sks}
 
 
-@pytest.mark.parametrize("N,S,M,parts", [(32, 96, 10, -1), (32, 96, 10, 8), (32, 96, 10, 0), (9, 30, 5, 2), (1, 0, 0, -1),
-                                          (2, 1, 1, -1), (17, 16, 0, 4)])
-def test_maximum_and_minimum_body_sizes(N, S, M, parts):
+# (N, S, M, WG_TUNE_PART, k_sub, obs layout).  The second list: one substep with the partition automatic (-1: off at
+# k_sub 1) or off, so the one-thread-per-env kernel is asked for, at the muscle counts around its shared-memory limit
+# (tile of 11 * N + M + 3 rows of 129 floats: at N = 32 on a B200 up to M = 92 with row-major, 95 with feature-major
+# observations); beyond it the step runs the mass-partitioned kernel with two lanes per env.  Which kernel ran is
+# checked in test_cuda_x64_bodies.py::test_float32_body_limit_kernels.
+BODY_SIZE_CASES = [(32, 96, 10, -1, 2, "row"), (32, 96, 10, 8, 2, "row"), (32, 96, 10, 0, 2, "row"), (9, 30, 5, 2, 2, "row"),
+                   (1, 0, 0, -1, 2, "row"), (2, 1, 1, -1, 2, "row"), (17, 16, 0, 4, 2, "row")]
+BODY_LIMIT_CASES = [(N, 96, M, parts, 1, layout) for N, M in ((32, 92), (32, 93), (32, 95), (32, 96), (16, 68))
+                    for parts in (-1, 0) for layout in ("row", "feature")]
+
+
+@pytest.mark.parametrize("N,S,M,parts,k_sub,layout", BODY_SIZE_CASES + BODY_LIMIT_CASES,
+                         ids=[f"{N}-{S}-{M}-{p}" for N, S, M, p, _, _ in BODY_SIZE_CASES] +
+                             [f"{N}-{S}-{M}-{p}-k{k}-{lay}" for N, S, M, p, k, lay in BODY_LIMIT_CASES])
+def test_maximum_and_minimum_body_sizes(N, S, M, parts, k_sub, layout):
     """The ABI limits (32 masses, 96 springs) and the degenerate ends (a single free mass, no muscles)
     on the generic and the mass-partitioned kernels, with float masses and a DingPoint."""
     import ctypes as C
@@ -360,10 +372,10 @@ def test_maximum_and_minimum_body_sizes(N, S, M, parts):
     old = lib.wg_set_tuning(_lib.TUNE_PART, parts)
     try:
         E = 300
-        env = BatchedPhysicsEnv(cr, E, "cuda:0", in3d=True, auto_reset="template", max_steps=5, k_sub=2, seed=3,
-                                keep_old_a=True, track_info=True, track_contacts=True, initial_reset=False)
+        env = BatchedPhysicsEnv(cr, E, "cuda:0", in3d=True, auto_reset="template", max_steps=5, k_sub=k_sub, seed=3,
+                                obs_layout=layout, keep_old_a=True, track_info=True, track_contacts=True, initial_reset=False)
         body = wo.make_body(spec)
-        prm = wo.make_params(in3d=True, auto_reset=2, max_steps=5, k_sub=2, seed=3)
+        prm = wo.make_params(in3d=True, auto_reset=2, max_steps=5, k_sub=k_sub, seed=3)
         st = wo.init_state(body, E)
         run_lockstep(env, body, prm, st, 9, rng, noise_reset=False)
     finally:
@@ -691,30 +703,41 @@ def test_rejected_step_leaves_the_bound_buffers_alone():
     assert gu.same(rew.cpu().numpy(), rew_r.cpu().numpy()) and float(out[0].min()) == 7.0 and float(out[1].min()) == 7.0
 
 
+def rope_bodies(rng):
+    """Balance-v0's graph (which has every specialisation) with two rope-type springs, and a random 9-mass body with a
+    mix of rope-type muscles and bones: [(points [(m, pos)], muscles [(i, j, kw)], skeletons [(i, j, kw)])]."""
+    base = [(5, (-50, 100, 0)), (5, (50, 100, 0)), (1, (0, 0, 0)), (3, (0, 100, 0))]
+    bodies = [(base, [(0, 2, {"string": True}), (1, 2, {})], [(0, 1, {}), (0, 3, {"string": True, "x": 60.0}), (1, 3, {})])]
+    pts9 = [(float(rng.integers(1, 6)), tuple(rng.uniform(-80, 80, 3).round(1))) for _ in range(9)]
+    pts9 = [(m, (p[0], abs(p[1]) + 5, p[2])) for m, p in pts9]
+    mus9 = [(int(i), int((i + 1 + rng.integers(0, 7)) % 9), {"string": bool(rng.integers(0, 2))}) for i in range(5)]
+    sks9 = [(int(i), int((i + 1) % 9), {"string": bool(rng.integers(0, 2)), "k": float(rng.choice([300, 1000, -500]))}) for i in range(9)]
+    bodies.append((pts9, [(i, j, kw) for i, j, kw in mus9 if i != j], [(i, j, kw) for i, j, kw in sks9 if i != j]))
+    return bodies
+
+
+def rope_creature(pts_s, mus_s, sks_s):
+    """(Creature, oracle spec) of one rope_bodies() entry; clears the Point registry first."""
+    from walker_gym_b200 import Creature, Muscle, Point, Skeleton
+    spec = {"points": [(m, p, False) for m, p in pts_s], "muscles": mus_s, "skeletons": sks_s}
+    Point.clear()
+    pts = [Point(m, list(p), [0, 0, 0]) for m, p in pts_s]
+    cr = Creature(pts, [Muscle(pts[i], pts[j], **kw) for i, j, kw in mus_s], [Skeleton(pts[i], pts[j], **kw) for i, j, kw in sks_s])
+    return cr, spec
+
+
 @pytest.mark.parametrize("E,layout,parts", [(1000, "row", -1), (777, "feature", -1), (515, "row", 4)])
 def test_rope_type_springs_match_oracle(E, layout, parts):
     """Rope-type springs (`string=True`, Point.resilience semantics, gym/optimized_engine.py:134-138) as a per-spring
     flag of the run-time-topology kernels: random bodies with a mix of rope-type muscles and bones, bit-exact against
     the oracle; a body with such springs never takes a compile-time specialisation."""
-    from walker_gym_b200 import BatchedPhysicsEnv, Creature, Muscle, Point, Skeleton, _lib
+    from walker_gym_b200 import BatchedPhysicsEnv, Point, _lib
     rng = np.random.default_rng(E)
     lib = _lib.load()
     old = lib.wg_set_tuning(_lib.TUNE_PART, parts)
-    Point.clear()
     try:
-        # Balance-v0's graph (which has every specialisation) with two rope-type springs, and a random 9-mass body
-        base = [(5, (-50, 100, 0)), (5, (50, 100, 0)), (1, (0, 0, 0)), (3, (0, 100, 0))]
-        bodies = [(base, [(0, 2, {"string": True}), (1, 2, {})], [(0, 1, {}), (0, 3, {"string": True, "x": 60.0}), (1, 3, {})])]
-        pts9 = [(float(rng.integers(1, 6)), tuple(rng.uniform(-80, 80, 3).round(1))) for _ in range(9)]
-        pts9 = [(m, (p[0], abs(p[1]) + 5, p[2])) for m, p in pts9]
-        mus9 = [(int(i), int((i + 1 + rng.integers(0, 7)) % 9), {"string": bool(rng.integers(0, 2))}) for i in range(5)]
-        sks9 = [(int(i), int((i + 1) % 9), {"string": bool(rng.integers(0, 2)), "k": float(rng.choice([300, 1000, -500]))}) for i in range(9)]
-        bodies.append((pts9, [(i, j, kw) for i, j, kw in mus9 if i != j], [(i, j, kw) for i, j, kw in sks9 if i != j]))
-        for pts_s, mus_s, sks_s in bodies:
-            spec = {"points": [(m, p, False) for m, p in pts_s], "muscles": mus_s, "skeletons": sks_s}
-            Point.clear()
-            pts = [Point(m, list(p), [0, 0, 0]) for m, p in pts_s]
-            cr = Creature(pts, [Muscle(pts[i], pts[j], **kw) for i, j, kw in mus_s], [Skeleton(pts[i], pts[j], **kw) for i, j, kw in sks_s])
+        for body_s in rope_bodies(rng):
+            cr, spec = rope_creature(*body_s)
             env = BatchedPhysicsEnv(cr, E, "cuda:0", in3d=True, auto_reset="template", max_steps=9, k_sub=2, seed=5,
                                     obs_layout=layout, keep_old_a=True, track_info=True, track_contacts=True, initial_reset=False)
             assert env.kernel_variant == 0 and env.state_layout == "soa"

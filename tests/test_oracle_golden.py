@@ -343,3 +343,59 @@ def test_rope_type_springs_follow_point_resilience():
             a2 = np.zeros(3, np.float32); a2 += (-force) / 3.0; a2 += damp / 3.0
             assert gu.same(got[:3, 0], a1) and gu.same(got[3:, 0], a2), (x, string)
         assert gu.same(outs[0], outs[1]) == (not slack)
+
+    # A rope-type muscle driven with float64 actions (wo.step_x64).  Its length is then an np.float64 ("strong") and the
+    # elastic term is NumPy float64 arithmetic: dx = np.float64(L) - x, f_size = -dx * float(k), a float64 force array,
+    # and Point.forced rounds `acc + force / m` once.  A length that regulation() clamped holds the float32 limit
+    # ("weak") and is back on the float32 arithmetic above.  The rope rule holds on both.
+    def muscle_spec(string, p2, x0, k):
+        return {"points": [(2.0, (0.0, 50.0, 0.0), False), (3.0, p2, False)], "skeletons": [],
+                "muscles": [(0, 1, {"x": x0, "k": k, "dampk": 12, "string": string})]}
+
+    def restated(string, p2, x0, k, a):
+        p1, p2 = np.array([0, 50, 0], np.float32), np.array(p2, np.float32)
+        v1, v2 = np.array([1, -2, 0.5], np.float32), np.array([-3, 4, 0.25], np.float32)
+        L = np.linalg.norm(p1 - p2)
+        direction = (p2 - p1) / L if L > 0 else p2 - p1         # coincident endpoints: no division (the oracle's guard)
+        x = np.float64(x0) + np.float64(a)                       # Muscle.x += a
+        lo, hi = x0 * 0.1, x0 * 1.5                              # originx a python float: python float limits
+        weak = bool(lo > x or hi < x)
+        if weak:
+            x = lo if lo > x else hi                             # max() / min() return the limit object
+            dx = L - x                                           # np.float32 - python float: float32
+            f_size = np.float32(0) if (string and dx < 0) else -dx * np.float32(k)
+            force = f_size * direction                           # float32
+        else:
+            dx = np.float64(L) - x
+            f_size = np.float64(0) if (string and dx < 0) else -dx * float(k)
+            force = np.float64(f_size) * direction.astype(np.float64)
+        damp = np.dot(v1 - v2, direction) * np.float32(12) * direction
+        a1 = np.zeros(3, np.float32); a1 += force / 2.0; a1 += (-damp) / np.float32(2.0)
+        a2 = np.zeros(3, np.float32); a2 += (-force) / 3.0; a2 += damp / np.float32(3.0)
+        return weak, np.concatenate([a1, a2])
+
+    cases = [  # (what, p2, x0, k, action, weak, slack); the endpoints are 50 apart unless p2 coincides with p1
+        ("strong slack", (30.0, 90.0, 0.0), 40.0, 700, 15.0, False, True),
+        ("strong taut", (30.0, 90.0, 0.0), 40.0, 700, -5.5, False, False),
+        ("strong slack, negative k", (30.0, 90.0, 0.0), 40.0, -700, 15.0, False, True),
+        ("weak slack", (30.0, 90.0, 0.0), 40.0, 700, 80.0, True, True),      # clamped to x0 * 1.5 = 60 > 50
+        ("weak taut", (30.0, 90.0, 0.0), 40.0, 700, -80.0, True, False),     # clamped to x0 * 0.1 = 4 < 50
+        ("L == x", (30.0, 90.0, 0.0), 40.0, 700, 10.0, False, False),        # dx = 0: f_size = -0 * k either way
+        ("coincident endpoints", (0.0, 50.0, 0.0), 40.0, 700, 3.0, False, True),
+    ]
+    for what, p2, x0, k, a, weak, slack in cases:
+        outs = []
+        for string in (False, True):
+            spec = muscle_spec(string, p2, x0, k)
+            body, xb = wo.make_body(spec), wo.make_x64(spec)
+            prm = wo.make_params(in3d=True, g=0, ground_high=-1000)
+            st = wo.init_state(body, 1)
+            st["mx64"], st["mx_weak"] = wo.init_x64(body, xb, 1)
+            st["vel"][:, 0] = np.array([1, -2, 0.5, -3, 4, 0.25], np.float32)
+            wo.step_x64(body, xb, prm, st, np.array([[a]], np.float64))
+            want_weak, want = restated(string, p2, x0, k, a)
+            assert want_weak == weak and int(st["mx_weak"][0, 0]) == int(weak), (what, string)
+            assert gu.same(st["old_a"][:, 0], want), (what, string, st["old_a"][:, 0], want)
+            outs.append(st["old_a"].copy())
+        # the flag changes the step exactly when the muscle is slack and its direction is defined
+        assert gu.same(outs[0], outs[1]) == (not slack or what == "coincident endpoints"), what

@@ -188,6 +188,14 @@ class BatchedPhysicsEnv:
         self._step_offset, self._defer_advance = 0, False
         self._buf = WgBuffers()
         self._bind()
+        if self.x64:
+            # a step of no envs checks the body: one too large for the x64 kernel is refused here, not at the first step
+            with torch.cuda.device(self.device):
+                rc = self.lib.wg_step_x64(C.byref(self.topo), C.byref(self._x64), C.byref(self.params),
+                                          C.byref(self._buf), 0, None)
+            if rc == -2:                        # WG_ERR_UNSUPPORTED
+                raise ValueError(self.lib.wg_last_error_string().decode("utf-8", "replace"))
+            _lib.check(rc, "wg_step_x64")
         if initial_reset:
             self.reset()           # PhysicsEnv.__init__ ends with self.reset() (gym/optimized_env.py:51)
 

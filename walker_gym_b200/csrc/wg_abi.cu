@@ -127,6 +127,7 @@ WG_MULTI_DECL(balance); WG_MULTI_DECL(box); WG_MULTI_DECL(legacy_box); WG_MULTI_
 WG_MULTI_DECL(hat); WG_MULTI_DECL(humanb); WG_MULTI_DECL(box4); WG_MULTI_DECL(leg2); WG_MULTI_DECL(leg);
 #undef WG_MULTI_DECL
 int launch_generic_step_x64(const wg_topology*, const wg_x64*, const wg_params*, const wg_buffers*, int64_t E, cudaStream_t);
+int check_generic_step_x64(const wg_topology*, const wg_params*, const wg_buffers*);
 int launch_pkg_update(const wg_pkg_system*, const wg_pkg_params*, float* pos, float* vel, float* old_a,
                       int64_t E, int32_t n_steps, bool force_generic, cudaStream_t);
 int pkg_variant(const wg_pkg_system*);
@@ -278,6 +279,8 @@ int wg_step_x64(const wg_topology* topo, const wg_x64* x64, const wg_params* prm
     if (buf->state_packed) return fail(WG_ERR_BAD_ARG, "x64 mode uses the SoA state layout%s");
     if (topo->n_muscle > 0 && (!buf->mx64 || !buf->mx_weak)) return fail(WG_ERR_BAD_ARG, "mx64 / mx_weak must be set%s");
     if (buf->act_dim > 0 && !buf->action64) return fail(WG_ERR_BAD_ARG, "action64 must be set when act_dim > 0%s");
+    rc = check_generic_step_x64(topo, prm, buf);               // also for n_env == 0: lets callers check a body up front
+    if (rc != WG_OK) return rc;
     if (n_env == 0) return WG_OK;
     return launch_generic_step_x64(topo, x64, prm, buf, n_env, (cudaStream_t)cuda_stream);
 }

@@ -1,8 +1,53 @@
 // wg_inst_generic.cu -- run-time-topology step kernel, reset kernel (K2), stats reduction (K3).
+#include <atomic>
+
 #include "wg_launch.cuh"
 namespace wg {
+// the per-env tile of the run-time-topology kernel: 11 * N + M + 3 rows of kBlock + 1 floats (x64 mode included)
 static size_t generic_smem(const wg_topology* t) {
     return sizeof(float) * (size_t)(11 * t->n_mass + t->n_muscle + 3) * (kBlock + 1);
+}
+
+// Dynamic shared memory a block of `kern` can have on the current device: the device's opt-in limit per block (queried
+// once per device) less the kernel's static shared memory.
+static int smem_room(const void* kern, size_t* room) {
+    constexpr int kMaxDevices = 64;
+    static std::atomic<int> optin[kMaxDevices];                 // 0 = not queried yet
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return fail(WG_ERR_CUDA, "cudaGetDevice: %s", cudaGetErrorString(e));
+    int lim = dev < kMaxDevices ? optin[dev].load(std::memory_order_relaxed) : 0;
+    if (lim == 0) {
+        e = cudaDeviceGetAttribute(&lim, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+        if (e != cudaSuccess) return fail(WG_ERR_CUDA, "cudaDeviceGetAttribute: %s", cudaGetErrorString(e));
+        if (dev < kMaxDevices) optin[dev].store(lim, std::memory_order_relaxed);
+    }
+    cudaFuncAttributes fa;
+    e = cudaFuncGetAttributes(&fa, kern);
+    if (e != cudaSuccess) return fail(WG_ERR_CUDA, "cudaFuncGetAttributes: %s", cudaGetErrorString(e));
+    *room = (size_t)lim > fa.sharedSizeBytes ? (size_t)lim - fa.sharedSizeBytes : 0;
+    return WG_OK;
+}
+
+// x64 mode has only the run-time-topology kernel: a body whose tile does not fit a block is refused
+template <bool IN3D, bool ROWMAJOR>
+static int check_generic_x64(const wg_topology* t) {
+    const size_t smem = generic_smem(t);
+    if (smem <= 48 * 1024) return WG_OK;
+    size_t room = 0;
+    const int rc = smem_room((const void*)step_generic_kernel<IN3D, ROWMAJOR, X64Args>, &room);
+    if (rc != WG_OK || smem <= room) return rc;
+    char msg[256];
+    snprintf(msg, sizeof(msg), "x64 mode: a body of %d masses and %d muscles needs %zu bytes of shared memory per block "
+             "(11 * n_mass + n_muscle + 3 rows of %d floats), this device allows %zu for the %s-observation kernel",
+             t->n_mass, t->n_muscle, smem, kBlock + 1, room, ROWMAJOR ? "row-major" : "feature-major");
+    return fail(WG_ERR_UNSUPPORTED, "%s", msg);
+}
+
+int check_generic_step_x64(const wg_topology* t, const wg_params* p, const wg_buffers* b) {
+    const bool rm = b->obs_layout == 0;
+    if (p->in3d) return rm ? check_generic_x64<true, true>(t) : check_generic_x64<true, false>(t);
+    return rm ? check_generic_x64<false, true>(t) : check_generic_x64<false, false>(t);
 }
 
 template <bool IN3D, bool ROWMAJOR>
@@ -16,7 +61,7 @@ static int launch_generic_x64(const wg_topology* t, const wg_x64* x, const wg_pa
     }
     XA.mx64 = b->mx64; XA.mx_weak = b->mx_weak; XA.action64 = b->action64;
     A.act_dim = b->action64 ? b->act_dim : 0;
-    const size_t smem = generic_smem(t) + sizeof(float) * (size_t)(3 * t->n_muscle) * (kBlock + 1);
+    const size_t smem = generic_smem(t);
     auto kern = step_generic_kernel<IN3D, ROWMAJOR, X64Args>;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -38,13 +83,19 @@ int launch_generic_step_x64(const wg_topology* t, const wg_x64* x, const wg_para
 template <bool IN3D, bool ROWMAJOR>
 static int launch_generic(const wg_topology* t, const wg_params* p, const wg_buffers* b, int64_t E, cudaStream_t s) {
     StepArgs<kMaxMass, kMaxSpring> A;
-    fill_args(A, t, p, b, E);
     const size_t smem = generic_smem(t);
     auto kern = step_generic_kernel<IN3D, ROWMAJOR, NoX64>;
     if (smem > 48 * 1024) {
+        // a tile too large for one block: the mass-partitioned kernel with two lanes per env computes the same bits
+        // with about half of it per block
+        size_t room = 0;
+        const int rc = smem_room((const void*)kern, &room);
+        if (rc != WG_OK) return rc;
+        if (smem > room) return launch_part_step(t, p, b, E, 2, s);
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return fail(WG_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     }
+    fill_args(A, t, p, b, E);
     const unsigned grid = (unsigned)((E + kBlock - 1) / kBlock);
     kern<<<grid, kBlock, smem, s>>>(A, NoX64{});
     cudaError_t e = cudaGetLastError();

@@ -421,33 +421,29 @@ step_generic_kernel(const __grid_constant__ StepArgs<kMaxMass, kMaxSpring> A, co
             st.base[(3 * N + r) * PITCH] = A.vel[(int64_t)r * E + e];
         }
         const int na = A.act_dim < M ? A.act_dim : M;
-        // x64 rows after the scratch rows: [0,M) low word, [M,2M) high word of the double length, [2M,3M) type bit
-        float* const xrow = st.base + (size_t)(11 * N + M + 3) * PITCH;
         uint32_t cp = 0;
         if constexpr (X64) {
+            // the post-action double lengths and type bits go back to their coalesced [M][E] arrays, which the substeps
+            // read: staged in shared memory they would cost 3M more rows and keep large bodies from launching
             for (int m = 0; m < M; m++) {
                 double x = XA.mx64[(int64_t)m * E + e];
-                uint32_t weak = XA.mx_weak[(int64_t)m * E + e];
                 if (m < na) {                                               // anything + np.float64 -> np.float64
                     x = x + (A.act_layout ? XA.action64[(int64_t)m * E + e] : XA.action64[e * A.act_dim + m]);
-                    weak = 0;
+                    uint8_t weak = 0;
                     if (XA.v.mlo_d[m] > x) { x = XA.v.mlo_d[m]; weak = 1; }   // max() returns the limit object
                     if (XA.v.mhi_d[m] < x) { x = XA.v.mhi_d[m]; weak = 1; }
+                    XA.mx64[(int64_t)m * E + e] = x;
+                    XA.mx_weak[(int64_t)m * E + e] = weak;
                 }
-                xrow[m * PITCH] = __int_as_float(__double2loint(x));
-                xrow[(M + m) * PITCH] = __int_as_float(__double2hiint(x));
-                xrow[(2 * M + m) * PITCH] = __uint_as_float(weak);
                 st.mx(m) = (float)x;                                        // float32 view: weak muscles, observation
             }
             for (int k = 0; k < A.ec.k_sub; k++) {
                 for (int n = 0; n < N; n++) { st.acc(n, 0) = 0.0f; st.acc(n, 1) = 0.0f; st.acc(n, 2) = 0.0f; }
                 for (int sp = 0; sp < M; sp++) {
-                    if (__float_as_uint(xrow[(2 * M + sp) * PITCH]))
+                    if (XA.mx_weak[(int64_t)sp * E + e])
                         spring_run<2>(topo, A.bv, st, sp, st.mx(sp), A.bv.fixed_mask);
                     else
-                        spring_run_x64(topo, A.bv, st, sp,
-                                       __hiloint2double(__float_as_int(xrow[(M + sp) * PITCH]), __float_as_int(xrow[sp * PITCH])),
-                                       XA.v.sk_d[sp], A.bv.fixed_mask);
+                        spring_run_x64(topo, A.bv, st, sp, XA.mx64[(int64_t)sp * E + e], XA.v.sk_d[sp], A.bv.fixed_mask);
                 }
                 for (int sp = M; sp < S; sp++) spring_run<2>(topo, A.bv, st, sp, A.bv.srest[sp], A.bv.fixed_mask);
                 cp = 0;
@@ -486,9 +482,8 @@ step_generic_kernel(const __grid_constant__ StepArgs<kMaxMass, kMaxSpring> A, co
             if constexpr (X64) {
                 if (A.ec.auto_reset == 2)                                   // a fresh Muscle: x = originx
                     for (int m = 0; m < M; m++) {
-                        xrow[m * PITCH] = __int_as_float(__double2loint(XA.v.x0_d[m]));
-                        xrow[(M + m) * PITCH] = __int_as_float(__double2hiint(XA.v.x0_d[m]));
-                        xrow[(2 * M + m) * PITCH] = __uint_as_float(1u);
+                        XA.mx64[(int64_t)m * E + e] = XA.v.x0_d[m];
+                        XA.mx_weak[(int64_t)m * E + e] = 1;
                     }
             }
         }
@@ -499,12 +494,6 @@ step_generic_kernel(const __grid_constant__ StepArgs<kMaxMass, kMaxSpring> A, co
             if (A.old_a) A.old_a[(int64_t)r * E + e] = st.base[(6 * N + r) * PITCH];
         }
         for (int m = 0; m < M; m++) A.mx[(int64_t)m * E + e] = st.mx(m);
-        if constexpr (X64) {
-            for (int m = 0; m < M; m++) {
-                XA.mx64[(int64_t)m * E + e] = __hiloint2double(__float_as_int(xrow[(M + m) * PITCH]), __float_as_int(xrow[m * PITCH]));
-                XA.mx_weak[(int64_t)m * E + e] = (uint8_t)__float_as_uint(xrow[(2 * M + m) * PITCH]);
-            }
-        }
         if (A.obs) {
             if (ROWMAJOR) {
                 // centroid of getstat (sequential sum, then / N) for the cooperative copy-out below

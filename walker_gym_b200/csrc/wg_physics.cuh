@@ -145,7 +145,8 @@ __device__ __forceinline__ void spring_run(const Topo& topo, const BV& bv, Store
     const float dx = L - x;
     float fs = (-dx) * bv.sk[sp];                                         // -dx * k (sign as written)
     // rope-type springs (`if dx < 0 and string: f_size = 0`, gym/optimized_engine.py:134-136): a per-spring flag of
-    // the run-time topology only -- bodies with such springs never reach the compile-time specialisations
+    // the run-time topology only -- bodies with such springs never reach the compile-time specialisations.  The rule
+    // holds for both action dtypes: spring_run_x64 applies it to the float64 length of a strong muscle
     if constexpr (!Topo::kStatic) { if (((bv.string_mask[sp >> 5] >> (sp & 31)) & 1u) && dx < 0.0f) fs = 0.0f; }
     const V3 F = v3_scale(d, fs);
     const V3 vd = v3_sub(v3(st.vel(i, 0), st.vel(i, 1), st.vel(i, 2)), v3(st.vel(j, 0), st.vel(j, 1), st.vel(j, 2)));
@@ -222,7 +223,9 @@ __device__ __forceinline__ void spring_run_x64(const Topo& topo, const BV& bv, S
     float d0 = pjx - pix, d1 = pjy - piy, d2 = pjz - piz;
     const float L = np_norm3(d0, d1, d2);
     div3_len(d0, d1, d2, L);
-    const double fs = (-((double)L - x)) * k_d;
+    const double dx = (double)L - x;
+    double fs = (-dx) * k_d;
+    if (((bv.string_mask[sp >> 5] >> (sp & 31)) & 1u) && dx < 0.0) fs = 0.0;   // rope-type, tested on the double dx
     const double F[3] = { fs * (double)d0, fs * (double)d1, fs * (double)d2 };
     const float dk = np_dot3(st.vel(i, 0) - st.vel(j, 0), st.vel(i, 1) - st.vel(j, 1),
                              st.vel(i, 2) - st.vel(j, 2), d0, d1, d2);
