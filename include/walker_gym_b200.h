@@ -17,7 +17,7 @@
  *   action          : row-major [E][act_dim] (act_layout 0) or feature-major [act_dim][E] (act_layout 1)
  *   obs             : row-major [E][D] (obs_layout 0) or feature-major [D][E] (obs_layout 1)
  *   reward [E], done uint8 [E], contact_* uint32 bitmask [E] (bit n = mass n)
- *   energy [E], centroid [3][E], ep_ret [E], fin_stats [4][E], nf_stats [2][E]
+ *   energy [E], centroid [3][E], ep_ret [E], fin_stats [4][E], nf_stats [2][E], truncated uint8 [E], final_obs like obs
  *   noise           : SoA like pos; already scaled by sigma
  * D = 3 * (in3d ? 3 : 2) * n_mass + n_muscle   (Creature.getstat, gym/optimized_walker.py:129-162)
  *
@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define WG_ABI_VERSION 4
+#define WG_ABI_VERSION 5
 #define WG_MAX_MASS 32
 #define WG_MAX_SPRING 96
 
@@ -165,6 +165,19 @@ typedef struct wg_buffers {
     float*       nf_stats;      /* in/out, optional: per-env sums over finished episodes whose return is not finite:
                                    [0] count, [1] length.  Such an episode then goes here instead of into fin_stats.
                                    Needs fin_stats and the running return (ep_ret, or state_packed) */
+    uint8_t*     truncated;     /* out, optional: [E], or [n_steps][E] in wg_step_multi.  1 iff done is set AND the time
+                                   limit fired (steps >= max_steps) AND none of the terminal clauses did: the fall
+                                   (mean y < fall_thresh), all masses stopped after step 100, and the non-finite reward
+                                   with end_nonfinite.  A step on which a terminal clause and the time limit coincide counts
+                                   as terminated (truncated = 0); terminated = done && !truncated.  done is unchanged.
+                                   Written for every env.  Not accepted by wg_step_host, wg_step_multi_host and
+                                   wg_policy_step */
+    float*       final_obs;     /* out, optional: laid out like obs (obs_layout), needs obs.  For every env whose done is
+                                   set this step, whatever the reset mode: the observation of the state the step ended
+                                   in, before any auto-reset -- exactly the bits obs would hold with auto_reset 0 (with
+                                   auto_reset 0 it equals obs).  Rows of envs that are not done are left untouched.
+                                   Rejected by wg_step_multi (which returns only the last observation), the host-buffer
+                                   calls and wg_policy_step */
 } wg_buffers;
 
 /*
@@ -446,6 +459,19 @@ int wg_policy_tc_status(void);
  */
 int wg_gae(const float* rewards, const float* values, const uint8_t* dones, float* advantages, float* returns,
            int32_t horizon, int64_t n_env, float gamma, float lam, float reward_clip, void* cuda_stream);
+
+/*
+ * wg_gae that bootstraps time-limit truncations (gymnasium's terminated / truncated split): truncated uint8 [T][n_env]
+ * (buf->truncated of the steps), final_values [T][n_env].  The value after step t is
+ *     done ? (truncated ? san(final_values[t]) : 0) : values[t+1],      san = the reward sanitiser,
+ * and the advantage carry is cut on every done, as in wg_gae.  final_values is read only where done and truncated are
+ * both set: other entries may hold anything, NaN included.  Passing final_values = values (the value of the state the
+ * truncated step started from) is the cheap approximation of legged_gym / rsl_rl.  With no truncated step and finite
+ * values the results are wg_gae's bits.
+ */
+int wg_gae_trunc(const float* rewards, const float* values, const uint8_t* dones, const uint8_t* truncated,
+                 const float* final_values, float* advantages, float* returns, int32_t horizon, int64_t n_env, float gamma,
+                 float lam, float reward_clip, void* cuda_stream);
 
 /*
  * Measurement aid (bench.py --probe-stream): n_threads threads each read vec_reads and write vec_writes 16-byte

@@ -10,7 +10,7 @@ import ctypes as C
 import os
 
 MAX_MASS, MAX_SPRING = 32, 96
-ABI_VERSION = 4
+ABI_VERSION = 5
 GEN_MAX_ROWS, GEN_MAX_MUSCLE = 32, 16
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -66,6 +66,8 @@ class WgBuffers(C.Structure):
         ("mx64", C.c_void_p), ("mx_weak", C.c_void_p), ("action64", C.c_void_p),      # x64 mode (wg_step_x64)
         ("action_gen", C.POINTER(WgActionGen)),                                         # wg_step_multi: in-kernel action source
         ("nf_stats", C.c_void_p),                                                       # [2][E] non-finite episodes
+        ("truncated", C.c_void_p),                                                      # [E] uint8: done by the time limit alone
+        ("final_obs", C.c_void_p),                                                      # like obs: pre-reset observation of done envs
     ]
 
 
@@ -103,7 +105,7 @@ TUNE_TMA, TUNE_PART, TUNE_L2_PREFETCH, TUNE_JIT, TUNE_POLICY_TC, TUNE_PDL = 0, 1
 EXPORTS = ("wg_abi_version", "wg_last_error_string", "wg_obs_dim", "wg_kernel_variant", "wg_force_generic",
            "wg_set_tuning", "wg_packed_state_floats", "wg_packed_available", "wg_jit_prepare",
            "wg_step", "wg_step_multi", "wg_step_x64", "wg_reset", "wg_stats_reduce", "wg_stats_reduce_split", "wg_step_host", "wg_step_multi_host", "wg_pkg_update_physics", "wg_pkg_kernel_variant",
-           "wg_policy_act", "wg_policy_step", "wg_gae", "wg_stream_probe", "wg_host_alloc", "wg_host_free", "wg_getstat", "wg_policy_tc_status",
+           "wg_policy_act", "wg_policy_step", "wg_gae", "wg_gae_trunc", "wg_stream_probe", "wg_host_alloc", "wg_host_free", "wg_getstat", "wg_policy_tc_status",
            "wg_selftest_div_smallint", "wg_selftest_forced_list", "wg_selftest_sqrt", "wg_selftest_div3")
 
 _lib = None
@@ -170,6 +172,8 @@ def load():
     lib.wg_stream_probe.restype = C.c_int
     lib.wg_gae.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int64,
                            C.c_float, C.c_float, C.c_float, C.c_void_p]
+    lib.wg_gae_trunc.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                 C.c_int32, C.c_int64, C.c_float, C.c_float, C.c_float, C.c_void_p]
     lib.wg_getstat.argtypes = [P(WgTopology), P(WgBuffers), C.c_void_p, C.c_int32, C.c_int32, C.c_float, C.c_float, C.c_float,
                                C.c_float, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p]
     lib.wg_getstat.restype = C.c_int
@@ -183,7 +187,7 @@ def load():
                  "wg_selftest_sqrt", "wg_selftest_div3"):
         getattr(lib, name).restype = C.c_int
     for name in ("wg_obs_dim", "wg_kernel_variant", "wg_force_generic", "wg_step", "wg_reset",
-                 "wg_stats_reduce", "wg_stats_reduce_split", "wg_step_host", "wg_pkg_update_physics", "wg_policy_act", "wg_gae"):
+                 "wg_stats_reduce", "wg_stats_reduce_split", "wg_step_host", "wg_pkg_update_physics", "wg_policy_act", "wg_gae", "wg_gae_trunc"):
         getattr(lib, name).restype = C.c_int
     _lib = lib
     return lib

@@ -74,7 +74,8 @@ class BatchedPhysicsEnv:
                  env_offset: int = 0, graph_safe: bool = False, integrator: str = "run1",
                  state_layout: str = "auto", x64: bool = False,
                  track_info: bool = False, track_stats: bool = True, track_contacts: bool = False,
-                 keep_old_a: bool = False, initial_reset: bool = True, nonfinite: str = "keep"):
+                 keep_old_a: bool = False, initial_reset: bool = True, nonfinite: str = "keep",
+                 track_truncation: bool = False):
         """``nonfinite`` decides what happens to an env whose state overflowed to inf / NaN (Balance-v0 as written does
         so a few dozen steps after a reset; such an env then steps NaN arithmetic until ``max_steps``):
           "keep"  -- the reference's semantics: nothing special; its episode return enters the statistics (and makes
@@ -84,7 +85,21 @@ class BatchedPhysicsEnv:
                      return statistics;
           "end"   -- as "count", and a step whose reward is not finite also sets ``done``, so the template auto-reset
                      (or the caller, with ``auto_reset="none"``) restarts the env.  Not with ``auto_reset="jitter"``:
-                     a jitter reset keeps the overflowed positions."""
+                     a jitter reset keeps the overflowed positions.
+
+        ``track_truncation=True`` tells time-limit truncation apart from termination (gymnasium's ``truncated`` /
+        ``terminated``): ``env.truncated`` (bool [E]) and ``step()``'s ``info["truncated"]`` are set for an env whose
+        episode ended this step because it reached ``max_steps`` while none of the terminal rules fired (the fall, all
+        masses stopped after step 100, and the non-finite reward under ``nonfinite="end"``); a step on which one of them
+        coincides with the time limit counts as terminated.  ``done`` is unchanged, and ``terminated = done & ~truncated``.
+        ``env.final_obs`` (zero-initialised, shaped like ``obs``; ``info["final_obs"]``) receives, for every env whose
+        ``done`` is set this step, the observation of the state the episode ended in, before any auto-reset (the bits
+        ``obs`` would hold with ``auto_reset="none"``); rows of envs that are not done are left as they were, so read
+        them only where ``done`` is set.  A tracking env always binds both buffers, so the fused policy + step kernel
+        (``RolloutCollector(fuse_step=True)``) falls back to its two launches, and ``step_host`` /
+        ``HostStepPipeline.submit*`` (the host-buffer step calls) refuse it when called.  ``step_many`` reports the flag
+        only into its ``truncated_out`` and writes no ``final_obs``.  Not provided: a truncated-episode count in
+        ``episode_stats()``."""
         if nonfinite not in NONFINITE:
             raise ValueError(f"nonfinite must be one of {NONFINITE}")
         if nonfinite != "keep" and not track_stats:
@@ -173,6 +188,9 @@ class BatchedPhysicsEnv:
         self.fin_stats = torch.zeros(4, E, dtype=f32, device=dev) if track_stats else None
         # [0] count, [1] length sum of finished episodes whose return is not finite ("count" / "end" only)
         self.nf_stats = torch.zeros(2, E, dtype=f32, device=dev) if nonfinite != "keep" else None
+        self._trunc_u8 = torch.zeros(E, dtype=torch.uint8, device=dev) if track_truncation else None
+        self.truncated = self._trunc_u8.view(torch.bool) if track_truncation else None
+        self.final_obs = torch.zeros_like(self.obs) if track_truncation else None
         self._stats_out = torch.zeros(8, dtype=torch.float64, device=dev)
         # graph_safe: the Philox step index lives in a device scalar advanced by a device op, so a
         # captured CUDA graph that replays step() keeps drawing fresh reset jitter
@@ -215,6 +233,7 @@ class BatchedPhysicsEnv:
         b.contact_pre, b.contact_post = self._p(self.contact_pre), self._p(self.contact_post)
         b.energy, b.centroid = self._p(self.energy), self._p(self.centroid)
         b.ep_ret, b.fin_stats, b.nf_stats = self._p(self._ep_ret), self._p(self.fin_stats), self._p(self.nf_stats)
+        b.truncated, b.final_obs = self._p(self._trunc_u8), self._p(self.final_obs)
         b.action, b.act_dim, b.noise = None, 0, None
         b.act_layout = 0 if self.act_layout == "row" else 1
         b.step_counter = self._p(self._counter)
@@ -381,12 +400,23 @@ class BatchedPhysicsEnv:
         ``out=(obs, reward, done)``: write this step's results straight into caller-owned tensors (e.g. slot t
         of a trajectory buffer) instead of the env's own buffers; ``done`` is uint8/bool.  The tensors may also be
         PINNED HOST memory (``walker_gym_b200.host.pinned_empty`` / ``tensor.pin_memory()``): the kernel then writes
-        observation rows, rewards and dones over PCIe itself, with no device staging buffer and no separate copy."""
+        observation rows, rewards and dones over PCIe itself, with no device staging buffer and no separate copy.
+        With ``track_truncation``: ``info["truncated"]`` (bool [E]) and ``info["final_obs"]`` (``env.final_obs``), and
+        ``out`` may carry a 4th entry, a 1-byte [E] destination for the flag."""
         b = self._buf
-        res_obs, res_rew, res_done = self.obs, self.reward, self.done
+        res_obs, res_rew, res_done, res_trunc = self.obs, self.reward, self.done, self.truncated
         # validate everything before touching the bound buffers: a rejected call must leave the env as it was
         if out is not None:
-            res_obs, res_rew, res_done = out
+            if len(out) not in (3, 4):
+                raise ValueError("out must be (obs, reward, done) or (obs, reward, done, truncated)")
+            if len(out) == 4 and self.truncated is None:
+                raise ValueError("out has a truncated entry: construct the env with track_truncation=True")
+            res_obs, res_rew, res_done = out[:3]
+            if len(out) == 4:
+                res_trunc = out[3]
+                if res_trunc.element_size() != 1 or res_trunc.numel() != self.num_envs or not res_trunc.is_contiguous() \
+                        or res_trunc.device != self.obs.device:
+                    raise ValueError("out truncated must be a contiguous 1-byte tensor of length num_envs on the env's device")
             self._check_f32(res_obs, self.obs.shape, "out obs", mapped_ok=True)
             self._check_f32(res_rew, (self.num_envs,), "out reward", mapped_ok=True)
             if res_done.element_size() != 1 or res_done.numel() != self.num_envs or not res_done.is_contiguous() \
@@ -410,6 +440,7 @@ class BatchedPhysicsEnv:
         b.action, b.action64, b.act_dim, b.noise = act_ptr, act64_ptr, act_dim, noise_ptr
         if out is not None:
             b.obs, b.reward, b.done = res_obs.data_ptr(), res_rew.data_ptr(), res_done.data_ptr()
+            b.truncated = self._p(res_trunc)
         self._stamp()
         try:
             with torch.cuda.device(self.device):
@@ -421,14 +452,18 @@ class BatchedPhysicsEnv:
         finally:
             b.noise = None
             b.obs, b.reward, b.done = self._p(self.obs), self._p(self.reward), self._p(self._done_u8)
+            b.truncated = self._p(self._trunc_u8)
         _lib.check(rc, "wg_step_x64" if self.x64 else "wg_step")
         self._advance()
         info = {}
         if self.energy is not None:
             info = {"steps": self.steps, "centroid_position": self.centroid, "total_energy": self.energy}
+        if res_trunc is not None:
+            info["truncated"], info["final_obs"] = res_trunc, self.final_obs
         return res_obs, res_rew, res_done, info
 
-    def step_many(self, actions: Optional[torch.Tensor], n_steps: Optional[int] = None, out=None, _host=None):
+    def step_many(self, actions: Optional[torch.Tensor], n_steps: Optional[int] = None, out=None, _host=None,
+                  truncated_out: Optional[torch.Tensor] = None):
         """``n_steps`` consecutive ``PhysicsEnv.step`` calls in ONE launch (``wg_step_multi``) for actions known up
         front: scripted gaits / open-loop controllers (the phase-table gait sketched at gym/walker.py:356-366), action repeat, replays.
 
@@ -439,7 +474,8 @@ class BatchedPhysicsEnv:
         Returns ``(obs, rewards [T, E], dones [T, E])``: ``obs`` is the observation after the last step (the env's own
         buffer), rewards / dones are per step.  Bit-identical to T ``step`` calls; needs ``state_layout="packed"``,
         row-major observations and actions, a body with an ahead-of-time packed kernel, and no per-step info buffers.
-        ``out=(rewards, dones)``: caller-owned result tensors (dones 1 byte per element)."""
+        ``out=(rewards, dones)``: caller-owned result tensors (dones 1 byte per element).  ``truncated_out``: an optional
+        1-byte [T, E] tensor that receives each step's truncation flag (see ``track_truncation``)."""
         if self.state is None or self.x64 or self.obs_layout != "row" or self.act_layout != "row":
             raise ValueError("step_many needs state_layout='packed', obs_layout='row', act_layout='row' and float32 actions")
         E = self.num_envs
@@ -481,11 +517,15 @@ class BatchedPhysicsEnv:
             self._check_f32(rew, (T, E), "out rewards")
             if done.element_size() != 1 or tuple(done.shape) != (T, E) or not done.is_contiguous():
                 raise ValueError("out dones must be a contiguous 1-byte tensor of shape [T, E]")
+        if truncated_out is not None and (truncated_out.element_size() != 1 or tuple(truncated_out.shape) != (T, E)
+                                          or not truncated_out.is_contiguous() or truncated_out.device != self.obs.device):
+            raise ValueError("truncated_out must be a contiguous 1-byte tensor of shape [T, E] on the env's device")
         b = self._buf
         saved = (b.old_a, b.contact_pre, b.contact_post, b.energy, b.centroid)
         b.old_a = b.contact_pre = b.contact_post = b.energy = b.centroid = None
         b.action, b.act_dim, b.noise = self._p(actions), (self.M if actions is not None else 0), None
         b.reward, b.done = rew.data_ptr(), done.data_ptr()
+        b.truncated, b.final_obs = self._p(truncated_out), None
         b.action_gen = C.pointer(gen) if gen is not None else None
         self._stamp()
         try:
@@ -498,6 +538,7 @@ class BatchedPhysicsEnv:
         finally:
             b.old_a, b.contact_pre, b.contact_post, b.energy, b.centroid = saved
             b.reward, b.done = self._p(self.reward), self._p(self._done_u8)
+            b.truncated, b.final_obs = self._p(self._trunc_u8), self._p(self.final_obs)
             b.action_gen = None
         _lib.check(rc, "wg_step_multi" if _host is None else "wg_step_multi_host")
         if self._counter is not None:
@@ -841,6 +882,8 @@ class StepGraph:
 
         g = StepGraph(env, actions)        # actions: device float32 [T, E, M]; overwrite in place between replays
         g.replay()                          # T steps; g.obs [T, E, D] (or the last one only), g.rewards / g.dones [T, E]
+
+    With ``track_truncation`` on the env, ``g.truncated`` [T, E] (uint8) receives each step's truncation flag.
     """
 
     def __init__(self, env: BatchedPhysicsEnv, actions: torch.Tensor, keep_obs: str = "last"):
@@ -856,6 +899,7 @@ class StepGraph:
         self.obs = torch.empty((n_obs,) + tuple(env.obs.shape), dtype=torch.float32, device=dev)
         self.rewards = torch.empty(self.T, E, dtype=torch.float32, device=dev)
         self.dones = torch.empty(self.T, E, dtype=torch.uint8, device=dev)
+        self.truncated = torch.empty(self.T, E, dtype=torch.uint8, device=dev) if env.truncated is not None else None
         snap = env.state_dict()                                   # warm-up outside capture, on a snapshot
         s = torch.cuda.Stream(device=dev)
         s.wait_stream(torch.cuda.current_stream(dev))
@@ -873,7 +917,8 @@ class StepGraph:
         with env.deferred_steps(self.T):
             for t in range(self.T):
                 env._step_offset = t
-                env.step(self.actions[t], out=(self.obs[t if self.obs.shape[0] > 1 else 0], self.rewards[t], self.dones[t]))
+                out = (self.obs[t if self.obs.shape[0] > 1 else 0], self.rewards[t], self.dones[t])
+                env.step(self.actions[t], out=out if self.truncated is None else out + (self.truncated[t],))
 
     def replay(self) -> None:
         self.graph.replay()

@@ -27,6 +27,9 @@ int launch_policy_step(const PolicyArgs& A, int precision, const wg_topology* t,
 int launch_stream_probe(const float* src, float* dst, int64_t n, int R, int W, cudaStream_t s);
 int launch_gae(const float* rewards, const float* values, const uint8_t* dones, float* adv, float* ret, int T, int64_t E,
                float gamma, float lam, float clip, cudaStream_t s);
+int launch_gae_trunc(const float* rewards, const float* values, const uint8_t* dones, const uint8_t* truncated,
+                     const float* final_values, float* adv, float* ret, int T, int64_t E, float gamma, float lam, float clip,
+                     cudaStream_t s);
 
 static thread_local char g_err[512] = "";
 static std::atomic<int> g_force_generic{0};
@@ -117,6 +120,7 @@ static int validate(const wg_topology* t, const wg_params* p, const wg_buffers* 
     } else if (!b->pos || !b->vel || !b->steps || (t->n_muscle > 0 && !b->mx))
         return fail(WG_ERR_BAD_ARG, "pos/vel/mx/steps must be set%s");
     if (b->obs_layout != 0 && b->obs_layout != 1) return fail(WG_ERR_BAD_ARG, "obs_layout must be 0 or 1%s");
+    if (b->final_obs && !b->obs) return fail(WG_ERR_BAD_ARG, "final_obs needs obs%s");
     if (b->act_layout != 0 && b->act_layout != 1) return fail(WG_ERR_BAD_ARG, "act_layout must be 0 or 1%s");
     if (b->action && b->act_dim < 0) return fail(WG_ERR_BAD_ARG, "act_dim < 0%s");
     return WG_OK;
@@ -241,6 +245,7 @@ int wg_step_multi(const wg_topology* topo, const wg_params* prm, const wg_buffer
     if (n_steps < 1 || n_steps > 65536) return fail(WG_ERR_BAD_ARG, "n_steps out of range [1, 65536]%s");
     if (n_action_steps != n_steps && n_action_steps != 1) return fail(WG_ERR_BAD_ARG, "n_action_steps must be n_steps or 1 (action repeat)%s");
     if (!buf->state_packed) return fail(WG_ERR_BAD_ARG, "wg_step_multi needs the packed state layout%s");
+    if (buf->final_obs) return fail(WG_ERR_BAD_ARG, "wg_step_multi returns only the last observation: final_obs must be null%s");
     if (buf->obs && buf->obs_layout != 0) return fail(WG_ERR_BAD_ARG, "wg_step_multi writes row-major observations%s");
     if (buf->action && (buf->act_layout != 0 || buf->act_dim != topo->n_muscle))
         return fail(WG_ERR_BAD_ARG, "wg_step_multi reads actions as [n_action_steps][n_env][n_muscle]%s");
@@ -307,6 +312,7 @@ int wg_step_host(const wg_topology* topo, const wg_params* prm, const wg_buffers
                  const float* h_action, float* h_obs, float* h_reward, uint8_t* h_done, void* cuda_stream) {
     int rc = validate(topo, prm, buf, n_env);
     if (rc != WG_OK) return rc;
+    if (buf->truncated || buf->final_obs) return fail(WG_ERR_BAD_ARG, "wg_step_host does not take buf->truncated / final_obs%s");
     cudaStream_t s = (cudaStream_t)cuda_stream;
     cudaError_t e = cudaSuccess;
     if (h_action) {
@@ -330,6 +336,7 @@ int wg_step_multi_host(const wg_topology* topo, const wg_params* prm, const wg_b
     int rc = validate(topo, prm, buf, n_env);
     if (rc != WG_OK) return rc;
     if (n_steps < 1 || (n_action_steps != n_steps && n_action_steps != 1)) return fail(WG_ERR_BAD_ARG, "bad n_steps / n_action_steps%s");
+    if (buf->truncated || buf->final_obs) return fail(WG_ERR_BAD_ARG, "wg_step_multi_host does not take buf->truncated / final_obs%s");
     cudaStream_t s = (cudaStream_t)cuda_stream;
     cudaError_t e = cudaSuccess;
     if (h_action) {
@@ -409,6 +416,8 @@ int wg_policy_step(const wg_mlp_policy* pol, const wg_topology* topo, const wg_p
     if (!body_ok || !prm->in3d || !buf->state_packed || buf->obs_layout != 0 || pol->obs_dim != 38 || pol->act_dim != 2 ||
         tuning(WG_TUNE_POLICY_TC) != 2)
         return fail(WG_ERR_UNSUPPORTED, "wg_policy_step: fused policy + step exists for Balance-v0 (3-D, packed state, row-major observations) with the tcgen05 pipeline%s");
+    if (buf->truncated || buf->final_obs)
+        return fail(WG_ERR_UNSUPPORTED, "wg_policy_step does not write buf->truncated / final_obs: make the two calls%s");
     if (n_env == 0) return WG_OK;
     PolicyArgs A;
     A.obs_layout = 0;
@@ -436,6 +445,17 @@ int wg_gae(const float* rewards, const float* values, const uint8_t* dones, floa
     if (horizon == 0 || n_env == 0) return WG_OK;
     return launch_gae(rewards, values, dones, advantages, returns, horizon, n_env, gamma, lam, reward_clip,
                       (cudaStream_t)cuda_stream);
+}
+
+int wg_gae_trunc(const float* rewards, const float* values, const uint8_t* dones, const uint8_t* truncated,
+                 const float* final_values, float* advantages, float* returns, int32_t horizon, int64_t n_env, float gamma,
+                 float lam, float reward_clip, void* cuda_stream) {
+    if (!rewards || !values || !dones || !truncated || !final_values || !advantages || !returns)
+        return fail(WG_ERR_BAD_ARG, "null argument%s");
+    if (horizon < 0 || n_env < 0) return fail(WG_ERR_BAD_ARG, "horizon / n_env < 0%s");
+    if (horizon == 0 || n_env == 0) return WG_OK;
+    return launch_gae_trunc(rewards, values, dones, truncated, final_values, advantages, returns, horizon, n_env, gamma, lam,
+                            reward_clip, (cudaStream_t)cuda_stream);
 }
 
 }  // extern "C"

@@ -155,4 +155,14 @@ int launch_gae(const float* rewards, const float* values, const uint8_t* dones, 
     return WG_OK;
 }
 
+int launch_gae_trunc(const float* rewards, const float* values, const uint8_t* dones, const uint8_t* truncated,
+                     const float* final_values, float* adv, float* ret, int T, int64_t E, float gamma, float lam, float clip,
+                     cudaStream_t s) {
+    gae_trunc_kernel<<<(unsigned)((E + 255) / 256), 256, 0, s>>>(rewards, values, dones, truncated, final_values, adv, ret, T, E,
+                                                                 gamma, lam, clip);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return fail(WG_ERR_CUDA, "gae (truncation) kernel launch: %s", cudaGetErrorString(e));
+    return WG_OK;
+}
+
 }  // namespace wg

@@ -35,11 +35,14 @@ struct StepArgs {
     int32_t pf_dist;          // packed kernel: L2 prefetch distance in tiles (0 = off)
     int32_t act_dim, act_layout;
     float* nf_stats;          // optional [2][E]: count and length sum of finished episodes whose return is not finite
+    uint8_t* truncated;       // optional [E] ([n_steps][E] in the multi-step kernel): 1 = done by the time limit alone
+    float* final_obs;         // optional, laid out like obs: the observation of a done env's state before any reset
 };
 
 // NF (template flag of the kernel families whose keep-mode code must stay exactly what it was, see
-// step_static_packed_kernel): false compiles the non-finite handling out -- the instance then ignores
-// ec.end_nonfinite and nf_stats, and the host launches it only when both are off.
+// step_static_packed_kernel): false compiles the non-finite handling, the truncation flag and the final observation
+// out -- the instance then ignores ec.end_nonfinite, nf_stats, truncated and final_obs, and the host launches it only
+// when all four are off.
 
 // ---- TMA 1-D bulk store helpers (shared memory -> global), used for the observation rows ----------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -88,12 +91,14 @@ __device__ __forceinline__ void st_vec(T* p, const T (&in)[EPT]) {
 #define WG_STF(ptr, arr) st_vec<EPT, float, typename Vec<EPT>::F>(ptr, arr)
 
 // ---- per-env epilogue: reward, done, info, stats, auto-reset (shared by both kernels) ----
-struct EpiOut { float reward; uint32_t cpost; int done; float energy; float cen[3]; };
+struct EpiOut { float reward; uint32_t cpost; int done; float energy; float cen[3]; int trunc; };
 
 // reward, done and info from the per-mass heights ys(i) and speeds sp(i) (already filled in)
+// want_trunc: compute EpiOut.trunc (the caller binds wg_buffers.truncated); otherwise it is 0
 template <bool NF = true, class BV, class Store, class YS, class SP>
 __device__ __forceinline__ void epilogue_reduce(int N, const BV& bv, const EnvConst& ec, Store& st, int32_t steps_now,
-                                                bool want_energy, bool want_centroid, YS ys, SP sp, EpiOut& o) {
+                                                bool want_energy, bool want_centroid, bool want_trunc, YS ys, SP sp,
+                                                EpiOut& o) {
     uint32_t cpost = 0; int ncon = 0;
 #pragma unroll
     for (int n = 0; n < N; n++)
@@ -118,6 +123,18 @@ __device__ __forceinline__ void epilogue_reduce(int N, const BV& bv, const EnvCo
     // height and speed, so an inf / NaN anywhere in the state reaches it in the same step.
     if (NF && ec.end_nonfinite && !is_finite(o.reward)) dn = 1;
     o.done = dn;
+    // truncation (wg_buffers.truncated): done because the time limit fired while none of the terminal clauses -- the
+    // fall, all masses stopped, the opt-in non-finite reward -- did.  _is_done stops at the time limit, so they are
+    // evaluated again here; a step on which one coincides with the time limit counts as terminated.
+    o.trunc = 0;
+    if (NF && want_trunc && steps_now >= ec.max_steps) {
+        bool all_stopped = true;
+#pragma unroll
+        for (int n = 0; n < N; n++) all_stopped = all_stopped && (sp(n) < 0.1f);
+        const bool term = (cy < ec.fall_thresh) || (all_stopped && steps_now > 100) ||
+                          (ec.end_nonfinite && !is_finite(o.reward));
+        o.trunc = term ? 0 : 1;
+    }
     if (want_energy) {                                           // _calculate_energy (:240-248)
         const float ke = np_pairwise_sum(N, [&](int i) { return bv.mass_f[i] * (sp(i) * sp(i)); });
         const float pe = np_pairwise_sum(N, [&](int i) { return bv.mg_f[i] * (ys(i) - ec.ground); });
@@ -152,9 +169,21 @@ __device__ __forceinline__ void account_episode(const Args& A, int64_t E, int64_
     A.fin_stats[3 * E + i] += 1.0f;
 }
 
+// final observation (wg_buffers.final_obs) of env i whose step set done: the observation of its state BEFORE any reset,
+// the bits obs would have held with auto_reset 0.  Stored straight to global memory, row-major ([E][D]) or
+// feature-major ([D][E]) like obs: such rows are sparse except when a synchronised batch hits its time limit.  Every
+// step kernel that keeps the whole state of an env in one thread calls this before apply_reset; the units kernel emits
+// the row lane by lane (step_units_kernel).
+template <bool IN3D, class Topo, class Args, class Store>
+__device__ __forceinline__ void store_final_obs(const Topo& topo, const Args& A, Store& st, int64_t E, int64_t i, bool rowmajor) {
+    const int64_t D = 3 * (IN3D ? 3 : 2) * topo.n() + topo.m();
+    float* const fo = A.final_obs;
+    get_obs<IN3D>(topo, A.bv.ndiv, st, [&](int k, float v) { if (rowmajor) fo[i * D + k] = v; else fo[(int64_t)k * E + i] = v; });
+}
+
 template <bool IN3D, bool NF = true, class Topo, class BV, class Store, class YS, class SP>
 __device__ __forceinline__ void epilogue(const Topo& topo, const BV& bv, const EnvConst& ec, Store& st,
-                                         int32_t steps_now, bool want_energy, bool want_centroid,
+                                         int32_t steps_now, bool want_energy, bool want_centroid, bool want_trunc,
                                          YS ys, SP sp, EpiOut& o) {
     const int N = topo.n();
 #pragma unroll
@@ -162,7 +191,7 @@ __device__ __forceinline__ void epilogue(const Topo& topo, const BV& bv, const E
         ys(n) = st.pos(n, 1);
         sp(n) = np_norm3(v3(st.vel(n, 0), st.vel(n, 1), st.vel(n, 2)));
     }
-    epilogue_reduce<NF>(N, bv, ec, st, steps_now, want_energy, want_centroid, ys, sp, o);
+    epilogue_reduce<NF>(N, bv, ec, st, steps_now, want_energy, want_centroid, want_trunc, ys, sp, o);
 }
 
 // =================================================================================
@@ -245,7 +274,7 @@ step_static_kernel(const __grid_constant__ Args A) {
                 }
             }
         }
-        float rew[EPT]; uint8_t dnb[EPT]; uint32_t cpre[EPT], cpost[EPT];
+        float rew[EPT]; uint8_t dnb[EPT], tnb[EPT]; uint32_t cpre[EPT], cpost[EPT];
         float eng[EPT], cen[3][EPT];
 #pragma unroll
         for (int j = 0; j < EPT; j++) {
@@ -269,9 +298,9 @@ step_static_kernel(const __grid_constant__ Args A) {
             const int32_t sn = stp[j] + 1;
             float ysr[N], spr[N];
             EpiOut o;
-            epilogue<IN3D>(topo, A.bv, A.ec, st[j], sn, A.energy != nullptr, A.centroid != nullptr,
+            epilogue<IN3D>(topo, A.bv, A.ec, st[j], sn, A.energy != nullptr, A.centroid != nullptr, A.truncated != nullptr,
                            [&](int i) -> float& { return ysr[i]; }, [&](int i) -> float& { return spr[i]; }, o);
-            rew[j] = o.reward; dnb[j] = (uint8_t)o.done; cpost[j] = o.cpost;
+            rew[j] = o.reward; dnb[j] = (uint8_t)o.done; tnb[j] = (uint8_t)o.trunc; cpost[j] = o.cpost;
             eng[j] = o.energy; cen[0][j] = o.cen[0]; cen[1][j] = o.cen[1]; cen[2][j] = o.cen[2];
             stp[j] = sn;
             if (A.ep_ret) {
@@ -279,6 +308,7 @@ step_static_kernel(const __grid_constant__ Args A) {
                 if (o.done) account_episode(A, E, e + j, r, sn);
                 epr[j] = (o.done && A.ec.auto_reset) ? 0.0f : r;
             }
+            if (o.done && A.final_obs) store_final_obs<IN3D>(topo, A, st[j], E, e + j, OBS == 1);
             if (o.done && A.ec.auto_reset) {
                 apply_reset<IN3D>(topo, A.bv, A.ec, st[j], A.ec.auto_reset, A.noise, E, e + j, step_index_of(A));
                 stp[j] = 0;
@@ -323,6 +353,7 @@ step_static_kernel(const __grid_constant__ Args A) {
         if (A.ep_ret) WG_STF(A.ep_ret + e, epr);
         if (A.reward) WG_STF(A.reward + e, rew);
         if (A.done) st_vec<EPT, uint8_t, typename Vec<EPT>::B>(A.done + e, dnb);
+        if (A.truncated) st_vec<EPT, uint8_t, typename Vec<EPT>::B>(A.truncated + e, tnb);
         if (A.contact_pre) st_vec<EPT, uint32_t, typename Vec<EPT>::U>(A.contact_pre + e, cpre);
         if (A.contact_post) st_vec<EPT, uint32_t, typename Vec<EPT>::U>(A.contact_post + e, cpost);
         if (A.energy) WG_STF(A.energy + e, eng);
@@ -462,11 +493,12 @@ step_generic_kernel(const __grid_constant__ StepArgs<kMaxMass, kMaxSpring> A, co
         }
         int32_t sn = A.steps[e] + 1;
         EpiOut o;
-        epilogue<IN3D>(topo, A.bv, A.ec, st, sn, A.energy != nullptr, A.centroid != nullptr,
+        epilogue<IN3D>(topo, A.bv, A.ec, st, sn, A.energy != nullptr, A.centroid != nullptr, A.truncated != nullptr,
                        [&](int i) -> float& { return st.scratch(M, i); },
                        [&](int i) -> float& { return st.scratch(M, N + i); }, o);
         if (A.reward) A.reward[e] = o.reward;
         if (A.done) A.done[e] = (uint8_t)o.done;
+        if (A.truncated) A.truncated[e] = (uint8_t)o.trunc;
         if (A.contact_pre) A.contact_pre[e] = cp;
         if (A.contact_post) A.contact_post[e] = o.cpost;
         if (A.energy) A.energy[e] = o.energy;
@@ -476,6 +508,7 @@ step_generic_kernel(const __grid_constant__ StepArgs<kMaxMass, kMaxSpring> A, co
             if (o.done) account_episode(A, E, e, r, sn);
             A.ep_ret[e] = (o.done && A.ec.auto_reset) ? 0.0f : r;
         }
+        if (o.done && A.final_obs) store_final_obs<IN3D>(topo, A, st, E, e, ROWMAJOR);
         if (o.done && A.ec.auto_reset) {
             apply_reset<IN3D>(topo, A.bv, A.ec, st, A.ec.auto_reset, A.noise, E, e, step_index_of(A));
             sn = 0;

@@ -57,7 +57,8 @@ __device__ __forceinline__ float gen_action(const ActionGen& G, int m, int32_t s
 // last step.
 // GEN: compile-time switch for the in-kernel action sources -- the tensor-action instance (GEN = false) stays exactly
 // the code it was (the loop is instruction-cache sensitive: a run-time branch around the generator cost it 6 %).
-// NF: as for step_static_packed_kernel (the non-finite handling compiled in; launched with it off only as NF = false).
+// NF: as for step_static_packed_kernel (the non-finite handling and the truncation flag compiled in; launched with all of
+// them off only as NF = false).
 template <class Topo, bool IN3D, int MM, class Args = StepArgs<Topo::N, Topo::S>, bool GEN = false, bool NF = true>
 __global__ void __launch_bounds__(kMultiBlock, multi_min_blocks(Topo::N))
 step_multi_packed_kernel(const __grid_constant__ Args A, const int n_steps, const int64_t act_stride,
@@ -135,7 +136,7 @@ step_multi_packed_kernel(const __grid_constant__ Args A, const int n_steps, cons
             const int32_t sn = stp + 1;
             float ysr[N], spr[N];
             EpiOut o;
-            epilogue<IN3D, NF>(topo, A.bv, A.ec, st, sn, false, false,
+            epilogue<IN3D, NF>(topo, A.bv, A.ec, st, sn, false, false, NF && A.truncated != nullptr,
                            [&](int i) -> float& { return ysr[i]; }, [&](int i) -> float& { return spr[i]; }, o);
             stp = sn;
             {
@@ -149,6 +150,7 @@ step_multi_packed_kernel(const __grid_constant__ Args A, const int n_steps, cons
             }
             if (A.reward) A.reward[(int64_t)t * E + e] = o.reward;
             if (A.done) A.done[(int64_t)t * E + e] = (uint8_t)o.done;
+            if (NF && A.truncated) A.truncated[(int64_t)t * E + e] = (uint8_t)o.trunc;
         }
 
         if (A.obs) {
@@ -207,7 +209,7 @@ inline int launch_multi_packed(const wg_topology* t, const wg_params* p, const w
     static thread_local ActionGen G;
     fill_gen(G, b);
     using SA = StepArgs<Topo::N, Topo::S>;
-    const bool nf = p->end_nonfinite || b->nf_stats;
+    const bool nf = p->end_nonfinite || b->nf_stats || b->truncated;
     auto kern = G.mode ? (nf ? step_multi_packed_kernel<Topo, IN3D, MM, SA, true, true> : step_multi_packed_kernel<Topo, IN3D, MM, SA, true, false>)
                        : (nf ? step_multi_packed_kernel<Topo, IN3D, MM, SA, false, true> : step_multi_packed_kernel<Topo, IN3D, MM, SA, false, false>);
     if (smem > 48 * 1024) {

@@ -23,8 +23,8 @@ static_assert(kPackedBlock % 128 == 0, "the packed layout is tiled by 128 envs")
 
 // Args: StepArgs<Topo::N, Topo::S> for the ahead-of-time specialisations; the run-time compiled ones (wg_jit.cu) take
 // the full-size StepArgs<kMaxMass, kMaxSpring> the host can fill for any body.
-// NF: the non-finite handling (wg_params.end_nonfinite, buf->nf_stats) is compiled in; the launcher takes the NF = false
-// instance when both are off, so the reference's semantics run exactly the code they ran before the option existed.
+// NF: the non-finite handling (wg_params.end_nonfinite, buf->nf_stats), the truncation flag (buf->truncated) and the
+// final observation (buf->final_obs) are compiled in; the launcher takes the NF = false instance when all four are off, so the reference's semantics run exactly the code they ran before the option existed.
 // MINB: resident CTAs per SM the compiler must allow (0 = the default for the body size).  The 7-CTA instance (72
 // registers) exists for grids that fit ONE wave at 7 CTAs per SM but not at 6 -- BASELINE config 3 as written, 2^20 envs
 // over 8 GPUs = 1024 CTAs per GPU against 148 x 6 = 888 slots: a second, 14 %-full wave would double the step time.
@@ -112,7 +112,7 @@ step_static_packed_kernel(const __grid_constant__ Args A) {
         const int32_t sn = stp + 1;
         float ysr[N], spr[N];
         EpiOut o;
-        epilogue<IN3D, NF>(topo, A.bv, A.ec, st, sn, A.energy != nullptr, A.centroid != nullptr,
+        epilogue<IN3D, NF>(topo, A.bv, A.ec, st, sn, A.energy != nullptr, A.centroid != nullptr, NF && A.truncated != nullptr,
                        [&](int i) -> float& { return ysr[i]; }, [&](int i) -> float& { return spr[i]; }, o);
         stp = sn;
         {   // episode statistics: the running return lives in the packed state
@@ -120,6 +120,7 @@ step_static_packed_kernel(const __grid_constant__ Args A) {
             if (o.done) account_episode<NF>(A, E, e, r, sn);
             epr = (o.done && A.ec.auto_reset) ? 0.0f : r;
         }
+        if (NF && o.done && A.final_obs) store_final_obs<IN3D>(topo, A, st, E, e, OBS == 1);
         if (o.done && A.ec.auto_reset) {
             apply_reset<IN3D>(topo, A.bv, A.ec, st, A.ec.auto_reset, A.noise, E, e, step_index_of(A));
             stp = 0;
@@ -147,6 +148,7 @@ step_static_packed_kernel(const __grid_constant__ Args A) {
         }
         if (A.reward) A.reward[e] = o.reward;
         if (A.done) A.done[e] = (uint8_t)o.done;
+        if (NF && A.truncated) A.truncated[e] = (uint8_t)o.trunc;
         if (A.contact_pre) A.contact_pre[e] = cp;
         if (A.contact_post) A.contact_post[e] = o.cpost;
         if (A.energy) A.energy[e] = o.energy;

@@ -154,11 +154,12 @@ step_part_kernel(const __grid_constant__ PartArgs PA) {
     if (valid && part == 0) {
         const int32_t sn = A.steps[e] + 1;
         EpiOut o;
-        epilogue_reduce(N, bv, A.ec, st, sn, A.energy != nullptr, A.centroid != nullptr,
+        epilogue_reduce(N, bv, A.ec, st, sn, A.energy != nullptr, A.centroid != nullptr, A.truncated != nullptr,
                         [&](int i) -> float& { return st.scratch(M, i); },
                         [&](int i) -> float& { return st.scratch(M, N + i); }, o);
         if (A.reward) A.reward[e] = o.reward;
         if (A.done) A.done[e] = (uint8_t)o.done;
+        if (A.truncated) A.truncated[e] = (uint8_t)o.trunc;
         if (A.contact_pre) A.contact_pre[e] = cpre;
         if (A.contact_post) A.contact_post[e] = o.cpost;
         if (A.energy) A.energy[e] = o.energy;
@@ -168,6 +169,7 @@ step_part_kernel(const __grid_constant__ PartArgs PA) {
             if (o.done) account_episode(A, E, e, r, sn);
             A.ep_ret[e] = (o.done && A.ec.auto_reset) ? 0.0f : r;
         }
+        if (o.done && A.final_obs) store_final_obs<IN3D>(topo, A, st, E, e, ROWMAJOR);   // the env's whole state is in st
         do_reset = (o.done && A.ec.auto_reset) ? 1 : 0;
         A.steps[e] = do_reset ? 0 : sn;
         if (do_reset && A.ec.auto_reset == 2)
@@ -383,10 +385,11 @@ step_units_kernel(const __grid_constant__ UnitsArgs<U, MM> UA) {
         const int32_t sn = A.steps[e] + 1;
         EpiOut o;
         ScratchPos sp{ scr + 2 * N };
-        epilogue_reduce(N, A.bv, A.ec, sp, sn, A.energy != nullptr, A.centroid != nullptr,
+        epilogue_reduce(N, A.bv, A.ec, sp, sn, A.energy != nullptr, A.centroid != nullptr, A.truncated != nullptr,
                         [&](int i) -> float& { return scr[i]; }, [&](int i) -> float& { return scr[N + i]; }, o);
         if (A.reward) A.reward[e] = o.reward;
         if (A.done) A.done[e] = (uint8_t)o.done;
+        if (A.truncated) A.truncated[e] = (uint8_t)o.trunc;
         if (A.contact_pre) A.contact_pre[e] = cpre;
         if (A.contact_post) A.contact_post[e] = o.cpost;
         if (A.energy) A.energy[e] = o.energy;
@@ -396,11 +399,47 @@ step_units_kernel(const __grid_constant__ UnitsArgs<U, MM> UA) {
             if (o.done) account_episode(A, E, e, r, sn);
             A.ep_ret[e] = (o.done && A.ec.auto_reset) ? 0.0f : r;
         }
-        do_reset = (o.done && A.ec.auto_reset) ? 1 : 0;
-        A.steps[e] = do_reset ? 0 : sn;
+        do_reset = (o.done ? 2 : 0) | ((o.done && A.ec.auto_reset) ? 1 : 0);
+        A.steps[e] = (do_reset & 1) ? 0 : sn;
     }
     (void)vmask;
     do_reset = __shfl_sync(0xffffffffu, do_reset, lane - u);
+    const bool ended = (do_reset & 2) != 0;
+    do_reset &= 1;
+    // this lane's entries of an observation row: masses m0 .. m0+U::N-1 and muscles g0 .. g0+U::M-1 (mid: the centroid)
+    auto emit_unit = [&](const float (&mid)[3], auto put) {
+#pragma unroll
+        for (int n = 0; n < U::N; n++) {
+            const int k0 = (m0 + n) * 3 * d;
+#pragma unroll
+            for (int c = 0; c < d; c++) {
+                put(k0 + c, rs.p_[n][c] - mid[c]);
+                put(k0 + d + c, rs.v_[n][c]);
+                put(k0 + 2 * d + c, rs.a_[n][c]);
+            }
+        }
+#pragma unroll
+        for (int m = 0; m < U::M; m++) put(3 * d * N + g0 + m, rs.mx(m));
+    };
+    auto centroid = [&]() {                             // getstat centroid: sequential sum over all masses, then / N
+        float mid[3] = { 0.0f, 0.0f, 0.0f };
+#pragma unroll
+        for (int n = 0; n < N; n++) { mid[0] = mid[0] + scr[2 * N + n * 3]; mid[1] = mid[1] + scr[2 * N + n * 3 + 1]; mid[2] = mid[2] + scr[2 * N + n * 3 + 2]; }
+        const ConstDiv nd = A.bv.ndiv;
+        scr[5 * N + 0] = div_const(mid[0], nd.m, nd.r, nd.kind);
+        scr[5 * N + 1] = div_const(mid[1], nd.m, nd.r, nd.kind);
+        scr[5 * N + 2] = div_const(mid[2], nd.m, nd.r, nd.kind);
+    };
+    if (A.final_obs) {                                  // the final row from the pre-reset state: each lane its own part
+        if (valid && ended && u == 0) centroid();
+        __syncwarp();
+        if (valid && ended) {
+            const float mid[3] = { scr[5 * N + 0], scr[5 * N + 1], scr[5 * N + 2] };
+            float* const fo = A.final_obs;
+            emit_unit(mid, [&](int k, float v) { if (ROWMAJOR) fo[e * D + k] = v; else fo[(int64_t)k * E + e] = v; });
+        }
+        __syncwarp();                                   // the centroid is read before the reset below moves the positions
+    }
     if (valid && do_reset) {                            // each lane resets its own unit (Philox keyed per global mass)
         const uint32_t si = step_index_of(A);
         UnitView<U> view{ rs, m0, g0 };
@@ -416,37 +455,14 @@ step_units_kernel(const __grid_constant__ UnitsArgs<U, MM> UA) {
             for (int c = 0; c < 3; c++) scr[2 * N + (m0 + n) * 3 + c] = rs.p_[n][c];
     }
     __syncwarp();
-    if (valid && A.obs) {
-        if (u == 0) {                                   // getstat centroid: sequential sum over all masses, then / N
-            float mid[3] = { 0.0f, 0.0f, 0.0f };
-#pragma unroll
-            for (int n = 0; n < N; n++) { mid[0] = mid[0] + scr[2 * N + n * 3]; mid[1] = mid[1] + scr[2 * N + n * 3 + 1]; mid[2] = mid[2] + scr[2 * N + n * 3 + 2]; }
-            const ConstDiv nd = A.bv.ndiv;
-            scr[5 * N + 0] = div_const(mid[0], nd.m, nd.r, nd.kind);
-            scr[5 * N + 1] = div_const(mid[1], nd.m, nd.r, nd.kind);
-            scr[5 * N + 2] = div_const(mid[2], nd.m, nd.r, nd.kind);
-        }
-    }
+    if (valid && A.obs && u == 0) centroid();
     __syncwarp();
     if (valid && A.obs) {
-        // this lane's entries of the observation row: masses m0 .. m0+U::N-1 and muscles g0 .. g0+U::M-1
         const float mid[3] = { scr[5 * N + 0], scr[5 * N + 1], scr[5 * N + 2] };
-        auto emit = [&](int k, float v) {
+        emit_unit(mid, [&](int k, float v) {
             if (ROWMAJOR) { if (OBS_BULK) otile[el * D + k] = v; else A.obs[e * D + k] = v; }
             else A.obs[(int64_t)k * E + e] = v;
-        };
-#pragma unroll
-        for (int n = 0; n < U::N; n++) {
-            const int k0 = (m0 + n) * 3 * d;
-#pragma unroll
-            for (int c = 0; c < d; c++) {
-                emit(k0 + c, rs.p_[n][c] - mid[c]);
-                emit(k0 + d + c, rs.v_[n][c]);
-                emit(k0 + 2 * d + c, rs.a_[n][c]);
-            }
-        }
-#pragma unroll
-        for (int m = 0; m < U::M; m++) emit(3 * d * N + g0 + m, rs.mx(m));
+        });
     }
     if (valid) {
         // ---- single HBM write of the state ----

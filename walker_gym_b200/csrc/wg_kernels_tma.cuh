@@ -83,7 +83,7 @@ __device__ __forceinline__ void env_compute_store(const Args& A, RegStore<Topo::
             const int32_t sn = stp + 1;
             float ysr[N], spr[N];
             EpiOut o;
-            epilogue<IN3D>(topo, A.bv, A.ec, st, sn, A.energy != nullptr, A.centroid != nullptr,
+            epilogue<IN3D>(topo, A.bv, A.ec, st, sn, A.energy != nullptr, A.centroid != nullptr, A.truncated != nullptr,
                            [&](int i) -> float& { return ysr[i]; }, [&](int i) -> float& { return spr[i]; }, o);
             stp = sn;
             if (A.ep_ret) {
@@ -91,6 +91,7 @@ __device__ __forceinline__ void env_compute_store(const Args& A, RegStore<Topo::
                 if (o.done) account_episode(A, E, e, r, sn);
                 A.ep_ret[e] = (o.done && A.ec.auto_reset) ? 0.0f : r;
             }
+            if (o.done && A.final_obs) store_final_obs<IN3D>(topo, A, st, E, e, OBS == 1);
             if (o.done && A.ec.auto_reset) {
                 apply_reset<IN3D>(topo, A.bv, A.ec, st, A.ec.auto_reset, A.noise, E, e, step_index_of(A));
                 stp = 0;
@@ -115,6 +116,7 @@ __device__ __forceinline__ void env_compute_store(const Args& A, RegStore<Topo::
             A.steps[e] = stp;
             if (A.reward) A.reward[e] = o.reward;
             if (A.done) A.done[e] = (uint8_t)o.done;
+            if (A.truncated) A.truncated[e] = (uint8_t)o.trunc;
             if (A.contact_pre) A.contact_pre[e] = cp;
             if (A.contact_post) A.contact_post[e] = o.cpost;
             if (A.energy) A.energy[e] = o.energy;

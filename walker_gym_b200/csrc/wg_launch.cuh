@@ -116,7 +116,7 @@ inline void fill_args(StepArgs<MAXN, MAXS>& A, const wg_topology* t, const wg_pa
     ec.max_steps = p->max_steps; ec.k_sub = p->k_sub; ec.auto_reset = p->auto_reset;
     ec.seed_lo = p->seed_lo; ec.seed_hi = p->seed_hi; ec.step_index = p->step_index; ec.env_offset = p->env_offset;
     ec.end_nonfinite = p->end_nonfinite;
-    A.nf_stats = b->nf_stats;
+    A.nf_stats = b->nf_stats; A.truncated = b->truncated; A.final_obs = b->final_obs;
     A.pos = b->pos; A.vel = b->vel; A.old_a = b->old_a; A.mx = b->mx; A.steps = b->steps;
     A.action = b->action; A.obs = b->obs; A.reward = b->reward; A.done = b->done;
     A.contact_pre = b->contact_pre; A.contact_post = b->contact_post; A.energy = b->energy; A.centroid = b->centroid;
@@ -216,7 +216,7 @@ inline int launch_static_packed(const wg_topology* t, const wg_params* p, const 
     constexpr bool bulk = (OBS == 1) && gcd_c(D, 32) <= 2;
     const size_t smem = (OBS == 1 && b->obs) ? sizeof(float) * kPackedBlock * (bulk ? D : (D | 1)) : 0;
     using SA = StepArgs<Topo::N, Topo::S>;
-    const bool nf = p->end_nonfinite || b->nf_stats;          // the non-finite handling is compiled into NF = true only
+    const bool nf = p->end_nonfinite || b->nf_stats || b->truncated || b->final_obs;   // compiled into NF = true only
     auto kern = nf ? step_static_packed_kernel<Topo, IN3D, OBS, MM, SA, true> : step_static_packed_kernel<Topo, IN3D, OBS, MM, SA, false>;
     const int64_t n_blocks = (E + kPackedBlock - 1) / kPackedBlock;
     if constexpr (Topo::N <= 4 && IN3D && OBS == 1 && (MM == 0 || MM == 3) && WG_PACKED_MIN_BLOCKS == 6 && WG_PACKED_BLOCK == 128) {

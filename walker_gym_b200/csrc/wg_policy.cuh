@@ -9,6 +9,7 @@
 //                       registers between layers: the k-slots of each MMA are permuted so that the accumulator
 //                       fragment of one layer IS the A fragment of the next (no shuffles, no shared memory).
 //   gae_kernel        : GAE(lambda) advantages / returns over a [T][E] trajectory, one thread per env.
+//   gae_trunc_kernel  : the same with time-limit truncations bootstrapped from a value of the final state.
 //
 // This is floating-point ML glue, not the bit-exact physics: it is checked against a plain PyTorch float32
 // reference with a stated tolerance (tests/test_cuda_policy.py).
@@ -385,6 +386,40 @@ gae_kernel(const float* __restrict__ rewards, const float* __restrict__ values, 
         a = delta + gamma * lam * nt * a;
         adv[(int64_t)t * E + e] = a;
         ret[(int64_t)t * E + e] = a + v;
+        vnext = v;
+    }
+}
+
+// GAE(lambda) that bootstraps time-limit truncations: the value after step t is V_{t+1} when the episode goes on, 0 when it
+// terminated, and final_values_t when it was truncated (a done step with truncated_t set); the advantage carry is cut on
+// every done.  final_values is sanitised like the rewards.  Selects only: final_values rows of the other envs are never
+// read into the arithmetic, so garbage there (NaN, inf) cannot leak.  With no truncated step and finite values
+// the bits are gae_kernel's.
+static __global__ void __launch_bounds__(256)
+gae_trunc_kernel(const float* __restrict__ rewards, const float* __restrict__ values, const uint8_t* __restrict__ dones,
+                 const uint8_t* __restrict__ truncated, const float* __restrict__ final_values, float* __restrict__ adv,
+                 float* __restrict__ ret, int T, int64_t E, float gamma, float lam, float clip) {
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= E) return;
+    float a = 0.0f, vnext = values[(int64_t)T * E + e];
+    for (int t = T - 1; t >= 0; t--) {
+        const int64_t i = (int64_t)t * E + e;
+        float r = rewards[i];
+        r = (r != r) ? 0.0f : fminf(fmaxf(r, -clip), clip);
+        const bool d = dones[i] != 0;
+        float boot = vnext;
+        if (d) {
+            boot = 0.0f;
+            if (truncated[i]) {
+                const float f = final_values[i];
+                boot = (f != f) ? 0.0f : fminf(fmaxf(f, -clip), clip);
+            }
+        }
+        const float v = values[i];
+        const float delta = r + gamma * boot - v;
+        a = d ? delta : delta + gamma * lam * a;
+        adv[i] = a;
+        ret[i] = a + v;
         vnext = v;
     }
 }

@@ -60,7 +60,7 @@ struct FusedStep {
         const int32_t sn = stp + 1;
         float ysr[N], spr[N];
         EpiOut o;
-        epilogue<IN3D>(topo, A.bv, A.ec, st, sn, A.energy != nullptr, A.centroid != nullptr,
+        epilogue<IN3D>(topo, A.bv, A.ec, st, sn, A.energy != nullptr, A.centroid != nullptr, false,
                        [&](int i) -> float& { return ysr[i]; }, [&](int i) -> float& { return spr[i]; }, o);
         stp = sn;
         {   // episode statistics: the running return lives in the packed state

@@ -76,6 +76,21 @@ class FusedPolicy:
         _lib.check(rc, "wg_policy_act")
 
 
+def gae_trunc(rewards, values, dones, truncated, final_values, advantages, returns, gamma: float, lam: float,
+              reward_clip: float) -> None:
+    """``wg_gae_trunc``: ``gae`` whose truncated steps (truncated [T, E], 1-byte) bootstrap from final_values [T, E]
+    instead of 0.  final_values is read only where a step is both done and truncated."""
+    T, E = rewards.shape
+    if values.shape != (T + 1, E) or dones.shape != (T, E) or truncated.shape != (T, E) or final_values.shape != (T, E) \
+            or dones.element_size() != 1 or truncated.element_size() != 1:
+        raise ValueError("gae_trunc: shape mismatch")
+    with torch.cuda.device(rewards.device):
+        rc = _lib.load().wg_gae_trunc(rewards.data_ptr(), values.data_ptr(), dones.data_ptr(), truncated.data_ptr(),
+                                      final_values.data_ptr(), advantages.data_ptr(), returns.data_ptr(), T, E, gamma, lam,
+                                      reward_clip, C.c_void_p(torch.cuda.current_stream(rewards.device).cuda_stream))
+    _lib.check(rc, "wg_gae_trunc")
+
+
 def gae(rewards, values, dones, advantages, returns, gamma: float, lam: float, reward_clip: float) -> None:
     """``wg_gae``: rewards [T, E], values [T+1, E], dones [T, E] (1-byte) -> advantages, returns [T, E]."""
     T, E = rewards.shape
@@ -118,11 +133,26 @@ class RolloutCollector:
     ``FeatureMajorMLP``) takes either layout; row-major observations (``obs_layout="row"``, the step kernel's fastest
     path) and row-major actions are the fastest combination.  The torch-op collector needs feature-major both.
     ``collect()`` returns views of device buffers: obs [T+1, D, E] (or [T+1, E, D]), actions [T, M, E] (or [T, E, M]),
-    logp/values/rewards [T(+1), E], dones [T, E]."""
+    logp/values/rewards [T(+1), E], dones [T, E].
+
+    ``bootstrap_truncated``: what the returns of an episode that hit ``max_steps`` bootstrap from.  ``None`` (default):
+    nothing -- every ``done`` is treated as termination, which biases the returns of time-limited episodes towards zero.
+    ``"final"``: the value of the state the episode ended in -- after each step a value-only policy pass over
+    ``env.final_obs`` fills ``final_values[t]`` -- the exact time-limit correction, at one extra value pass per step.
+    ``"current"``: the value V(s_t) of the state the truncated step started from (legged_gym / rsl_rl's approximation; no
+    extra policy pass).  Both need ``BatchedPhysicsEnv(track_truncation=True)``; ``collect()`` then adds ``truncated``
+    [T, E] and, for ``"final"``, ``final_values`` [T, E] (rows of steps that are not done hold whatever the value pass made
+    of stale observations; GAE never reads them)."""
 
     def __init__(self, env: BatchedPhysicsEnv, policy: torch.nn.Module, horizon: int, *, gamma: float = 0.99,
                  lam: float = 0.95, use_cuda_graph: bool = True, reward_clip: float = 1e3, fused: Optional[bool] = None,
-                 precision: str = "fp32", seed: int = 0, fuse_step: bool = False):
+                 precision: str = "fp32", seed: int = 0, fuse_step: bool = False,
+                 bootstrap_truncated: Optional[str] = None):
+        if bootstrap_truncated not in (None, "current", "final"):
+            raise ValueError("bootstrap_truncated must be None, 'current' or 'final'")
+        if bootstrap_truncated is not None and env.truncated is None:
+            raise ValueError("bootstrap_truncated needs BatchedPhysicsEnv(track_truncation=True)")
+        self.bootstrap_truncated = bootstrap_truncated
         row = env.obs_layout == "row" or env.act_layout == "row"
         if row and fused is False:
             raise ValueError("the torch-op collector needs obs_layout='feature' and act_layout='feature'")
@@ -138,6 +168,8 @@ class RolloutCollector:
         self.values = torch.zeros(self.T + 1, E, **f32)
         self.rewards = torch.zeros(self.T, E, **f32)
         self.dones = torch.zeros(self.T, E, dtype=torch.bool, device=dev)
+        self.truncated = torch.zeros(self.T, E, dtype=torch.bool, device=dev) if bootstrap_truncated else None
+        self.final_values = torch.zeros(self.T, E, **f32) if bootstrap_truncated == "final" else None
         self.advantages = torch.zeros(self.T, E, **f32)
         self.returns = torch.zeros(self.T, E, **f32)
         self._graph: Optional[torch.cuda.CUDAGraph] = None
@@ -151,13 +183,15 @@ class RolloutCollector:
         self._fp = FusedPolicy(policy, precision) if self.fused else None
         self.seed = int(seed)
         # fuse_step=True: one launch per env step where the library has the env step fused into the policy pipeline
-        # (wg_policy_step: Balance-v0, 3-D, packed state, row-major observations / actions; probed with an empty call).
+        # (wg_policy_step: Balance-v0, 3-D, packed state, row-major observations / actions, no truncation flag; probed
+        # with an empty call).
         # Bit-identical to the two launches but measured SLOWER on B200 (71 vs 53 us per 2^18-env step: the output warps
         # that carry the step run its long straight-line body almost alone on their schedulers), hence off by default --
         # see DESIGN.md, K5.
         self.fused_step = bool(self.fused and fuse_step and not env.x64 and env.state_layout == "packed"
                                and env.obs_layout == "row" and env.act_layout == "row" and self._policy_step(0, probe=True))
-        self.kernel_launches_per_rollout = ((self.T if self.fused_step else 2 * self.T) + 2) if self.fused else self.T   # ours only
+        self.kernel_launches_per_rollout = ((self.T if self.fused_step else 2 * self.T) + 2 +
+                                            (self.T if bootstrap_truncated == "final" else 0)) if self.fused else self.T   # ours only
 
     def _policy_step(self, t: int, probe: bool = False) -> bool:
         """``wg_policy_step``: policy evaluation of ``obs[t]`` + ``env.step`` with the sampled action in ONE launch; results
@@ -203,10 +237,18 @@ class RolloutCollector:
                     continue
                 fp.act(self.obs[t], action=self.actions[t], logp=self.logp[t], value=self.values[t], sample=True,
                        step_index=t if env._counter is not None else env.step_count, **kw)
-                env.step(self.actions[t], out=(self.obs[t + 1], self.rewards[t], dones_u8[t]))
+                out = (self.obs[t + 1], self.rewards[t], dones_u8[t])
+                env.step(self.actions[t], out=out if self.truncated is None else out + (self.truncated[t],))
+                if self.final_values is not None:        # "final": the value of the state each ended episode ended in
+                    fp.act(env.final_obs, value=self.final_values[t], sample=False, **kw)
         fp.act(self.obs[self.T], value=self.values[self.T], sample=False, **kw)
         env.obs.copy_(self.obs[self.T])                  # keep env.obs current for the next rollout / other callers
-        gae(self.rewards, self.values, dones_u8, self.advantages, self.returns, self.gamma, self.lam, self.reward_clip)
+        if self.truncated is None:
+            gae(self.rewards, self.values, dones_u8, self.advantages, self.returns, self.gamma, self.lam, self.reward_clip)
+        else:                                            # a truncated step bootstraps from V(final state) or V(s_t)
+            fv = self.final_values if self.final_values is not None else self.values[: self.T]
+            gae_trunc(self.rewards, self.values, dones_u8, self.truncated.view(torch.uint8), fv,
+                      self.advantages, self.returns, self.gamma, self.lam, self.reward_clip)
 
     @torch.no_grad()
     def _rollout(self) -> None:
@@ -221,7 +263,11 @@ class RolloutCollector:
             act = torch.addcmul(mean, std, eps, out=self.actions[t])
             self.logp[t] = (-0.5 * eps * eps - pol.log_std - 0.5 * math.log(2 * math.pi)).sum(0)
             self.values[t] = value
-            obs, rew, done, _ = env.step(act)
+            obs, rew, done, info = env.step(act)
+            if self.truncated is not None:
+                self.truncated[t] = info["truncated"]
+            if self.final_values is not None:
+                self.final_values[t] = pol(env.final_obs)[1]
             self.obs[t + 1].copy_(obs)
             r = torch.nan_to_num(rew, nan=0.0, posinf=self.reward_clip, neginf=-self.reward_clip)
             self.rewards[t] = r.clamp_(-self.reward_clip, self.reward_clip)
@@ -231,7 +277,13 @@ class RolloutCollector:
         adv = torch.zeros_like(self.values[0])
         for t in range(self.T - 1, -1, -1):
             nonterminal = (~self.dones[t]).to(torch.float32)
-            delta = self.rewards[t] + self.gamma * self.values[t + 1] * nonterminal - self.values[t]
+            if self.truncated is None:
+                delta = self.rewards[t] + self.gamma * self.values[t + 1] * nonterminal - self.values[t]
+            else:                                        # a truncated step bootstraps from V(final state) or V(s_t)
+                fv = self.final_values[t] if self.final_values is not None else self.values[t]
+                final = torch.nan_to_num(fv, nan=0.0).clamp(-self.reward_clip, self.reward_clip)
+                boot = torch.where(self.dones[t], torch.where(self.truncated[t], final, 0.0), self.values[t + 1])
+                delta = self.rewards[t] + self.gamma * boot - self.values[t]
             adv = delta + self.gamma * self.lam * nonterminal * adv
             self.advantages[t] = adv
         torch.add(self.advantages, self.values[: self.T], out=self.returns)
@@ -255,8 +307,13 @@ class RolloutCollector:
                 with torch.cuda.graph(self._graph):
                     self._rollout()
             self._graph.replay()
-        return {"obs": self.obs, "actions": self.actions, "logp": self.logp, "values": self.values,
-                "rewards": self.rewards, "dones": self.dones, "advantages": self.advantages, "returns": self.returns}
+        out = {"obs": self.obs, "actions": self.actions, "logp": self.logp, "values": self.values,
+               "rewards": self.rewards, "dones": self.dones, "advantages": self.advantages, "returns": self.returns}
+        if self.truncated is not None:
+            out["truncated"] = self.truncated
+        if self.final_values is not None:
+            out["final_values"] = self.final_values
+        return out
 
     def episode_stats(self, all_reduce: bool = True) -> dict:
         """Finished-episode return statistics of all ranks: K3 reduction + one NCCL all-reduce of 8 doubles.  Also the
